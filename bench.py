@@ -2,6 +2,7 @@
 """bench.py — message-passing edges/s (fwd+bwd) of the GMLM GNN-encoder hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c4|c5|c2|c3]
+                    [--dump-outputs DIR]
 
 One "step" = one forward + one backward propagate of the F=256 RGCN mean aggregation (the
 kernel pair SURVEY §8(d) defines the algorithmic bytes for: 1162 B/edge in bf16) over the whole
@@ -65,6 +66,28 @@ def _ones_like(y):
             _ONES_CACHE.clear()
         t = _ONES_CACHE[key] = torch.ones_like(y)
     return t
+
+
+DUMP_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, outputs):
+    """Write each output of the timed path as <out_dir>/<name>.npy in float32.  An output larger than its share of
+    DUMP_BYTES keeps a fixed sample of rows (one row drawn by a seeded CPU generator from each of k equal strides):
+    the same rows for every run with the same arguments, so two builds can be compared output for output."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    share = DUMP_BYTES // len(outputs)
+    for name, t in outputs.items():
+        rows, width = t.shape[0], t[0].numel() if t.shape[0] else 1
+        k = min(rows, max(1, share // (4 * width)))
+        if k < rows:
+            stride = rows // k
+            idx = torch.arange(k) * stride + torch.randint(0, stride, (k,), generator=torch.Generator().manual_seed(0))
+            t = t[idx.to(t.device)]
+        np.save(out_dir / f"{name}.npy", t.float().cpu().numpy())
+        print(f"dumped {name}: {k} of {rows} rows, float32", file=sys.stderr, flush=True)
 
 
 class ClockSampler:
@@ -226,8 +249,9 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------- our arm, one GPU
-def measure_single(args, key: str, extras: bool, with_cpu: bool):
-    """One workload on one GPU -> the fields of the JSON line (value, roofline, e2e, context legs)."""
+def measure_single(args, key: str, extras: bool, with_cpu: bool, dump_dir=None):
+    """One workload on one GPU -> the fields of the JSON line (value, roofline, e2e, context legs).  With
+    ``dump_dir``, the last timed step's outputs are written there (dump_outputs)."""
     import gmlm_b200 as G
     from gmlm_b200 import _lib, synth
 
@@ -298,6 +322,8 @@ def measure_single(args, key: str, extras: bool, with_cpu: bool):
     torch.cuda.synchronize()
     torch.cuda.nvtx.range_pop()
     clocks = sampler.stop()
+    if dump_dir is not None:
+        dump_outputs(dump_dir, {"h": h, "grad_x": gx})
     total_ms = t_start.elapsed_time(t_end)
     ms_per_step = total_ms / args.steps
     fwd_all = [a.elapsed_time(b) for a, b, _ in ev]
@@ -598,9 +624,10 @@ def run_single(args):
     denominator of the 1/2/4/8-GPU scaling the metric names — followed by configs[3] (2M / 40M, the
     HBM-roofline study, with the layer / encoder / stock-torch context legs) under the key "c4"."""
     if args.workload != "c5":
-        print(json.dumps(measure_single(args, args.workload, extras=True, with_cpu=True)), flush=True)
+        print(json.dumps(measure_single(args, args.workload, extras=True, with_cpu=True, dump_dir=args.dump_outputs)),
+              flush=True)
         return
-    line = measure_single(args, "c5", extras=False, with_cpu=False)
+    line = measure_single(args, "c5", extras=False, with_cpu=False, dump_dir=args.dump_outputs)
     if not args.no_c4:
         c4 = measure_single(args, "c4", extras=True, with_cpu=True)
         line["cpu_baseline"] = c4.pop("cpu_baseline")          # bounded R-MAT sample: the same for both graphs
@@ -1068,9 +1095,16 @@ def main():
     ap.add_argument("--no-small", action="store_true", help="N=1 default run: skip the configs[1]/[2] (C2/C3) legs")
     ap.add_argument("--cpu-sample-nodes", type=int, default=100_000)
     ap.add_argument("--cpu-sample-edges", type=int, default=2_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="N=1: write the last timed step's outputs (h, grad_x) to DIR/<name>.npy, float32, a fixed "
+                         "row sample when larger than %d MiB in all" % (DUMP_BYTES >> 20))
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or max(args.gpus, world) > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.workload is None:
         args.workload = "c5"          # same graph at every N: the driver's scaling ratio compares like with like
     if args.impl == "reference":

@@ -44,3 +44,24 @@ def test_algorithmic_bytes_match_survey_8d():
     assert abs((fwd + bwd) / 40_000_000 - 1162) < 1                                 # 1162 B/edge
     fwd5, bwd5 = bench.algorithmic_bytes(10_000_000, 200_000_000, 256, 2, 4)        # C5
     assert abs((fwd5 + bwd5) / 1e9 - 232.4) < 0.1                                   # "232.4 GB" whole graph on 1 GPU
+
+
+def test_dump_outputs_is_float32_bounded_and_samples_the_same_rows(tmp_path):
+    """--dump-outputs: a large output is cut to a fixed row sample within the byte budget, a small one is kept
+    whole, everything is float32, and a second dump of the same tensors is identical."""
+    import numpy as np
+    import torch
+    import bench
+    big = torch.randn(3_000_000, 8).bfloat16()                 # 96 MB as float32: over the budget
+    small = torch.randn(100, 8)
+    for d in ("a", "b"):
+        bench.dump_outputs(tmp_path / d, {"h": big, "grad_x": small})
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["grad_x.npy", "h.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES + 4096
+    h = np.load(tmp_path / "a" / "h.npy")
+    assert h.dtype == np.float32 and 0 < h.shape[0] < big.shape[0] and h.shape[1] == 8
+    assert np.array_equal(h, np.load(tmp_path / "b" / "h.npy"))
+    for r in (h[0], h[-1]):                                    # whole rows of the output, not mixed values
+        assert bool((big.float() == torch.from_numpy(r)).all(1).any())
+    assert np.array_equal(np.load(tmp_path / "a" / "grad_x.npy"), small.numpy())
