@@ -7,9 +7,16 @@
 // dimension, every thread owns a fixed pack of channels and strides over rows, so the
 // per-channel constants live in registers.  Column reductions are two-stage and
 // order-fixed (per-CTA fp64 partials, then one in-order pass): no atomics, run-to-run
-// deterministic, and the fp64 accumulation makes the one-pass variance
-//   E[(x - a*mu)^2] = E[x^2] - mu^2 * (2a - a^2)
-// as accurate as the reference's two-pass form.
+// deterministic.  The variance is one-pass,
+//   E[(x - a*mu)^2] = (sum x^2 - sum x * mu * (2a - a^2)) / N,
+// which cancels when the column's offset is large against its spread (worst at a = 1, PyG's init).
+// For fp32 activations the column sums are therefore taken about a pivot, the column's first row p:
+// d = x - p (exact), d^2 (one fp64 rounding) and both sums are formed in fp64, and sum x = sum d + N p,
+// sum x^2 = sum d^2 + 2 p sum d + N p^2 are rebuilt once per column at the end.  A constant column
+// then gives sum x^2 == fl(sum x * mu) bit for bit, so its variance is exactly 0 and rstd exactly
+// 1/sqrt(eps); an offset column keeps about the two-pass form's accuracy up to offset/spread ~ 1e3,
+// beyond which the fp32 mean the forward stores is the limit.  bf16 activations (8-bit mantissa, exact
+// squares in fp32) keep fp32 running sums per thread.
 #include <algorithm>
 
 #include <type_traits>
@@ -93,23 +100,54 @@ __device__ __forceinline__ float gelu_grad_f(float n) {
 }
 
 // ---------------------------------------------------------------- column sums
-// partial[(by * 2 + k) * C + c], k = 0: sum, k = 1: sum of squares.  Optional row mask.
+// partial[(by * 2 + k) * C + c], k = 0: sum, k = 1: sum of squares; for fp32 taken about pivot[c] when
+// pivot is given (colstats_final_kernel adds it back).  Optional row mask.
 template <typename T, int VEC>
 __global__ void __launch_bounds__(kCta) colstats_kernel(const T* __restrict__ x, int64_t num_rows, int64_t C,
-                                                        int64_t ldx, const uint8_t* __restrict__ mask, int tpr,
+                                                        int64_t ldx, const uint8_t* __restrict__ mask,
+                                                        const float* __restrict__ pivot, int tpr,
                                                         double* __restrict__ partial) {
   __shared__ double sh[2][kCta];
   const int tx = threadIdx.x % tpr, ty = threadIdx.x / tpr, rpc = kCta / tpr;
   const int64_t cp = int64_t(blockIdx.x) * tpr + tx;
   const int64_t c0 = cp * VEC;
   const bool cvalid = c0 < C;
-  // per-thread running sums: fp64 for fp32 activations (the 1e-5 gate); bf16 activations (resolution 4e-3, ~100
-  // rows per thread) keep them in fp32 and widen only for the cross-thread / cross-CTA reduction
+  // per-thread running sums: fp64 for fp32 activations; bf16 activations (resolution 4e-3, ~100 rows per
+  // thread) keep them in fp32 and widen only for the cross-thread / cross-CTA reduction
   using AccT = typename std::conditional<sizeof(T) == 2, float, double>::type;
   AccT s[VEC], q[VEC];
 #pragma unroll
   for (int k = 0; k < VEC; ++k) s[k] = q[k] = AccT(0);
-  if (cvalid) {
+  if constexpr (sizeof(T) == 4) {
+    if (cvalid) {
+      double p[VEC];
+#pragma unroll
+      for (int k = 0; k < VEC; ++k) p[k] = pivot ? double(pivot[c0 + k]) : 0.0;
+      const int64_t stride = int64_t(gridDim.y) * rpc;
+      for (int64_t r = int64_t(blockIdx.y) * rpc + ty; r < num_rows; r += stride * kU) {
+        Pack<T, VEC> v[kU];
+        bool ok[kU];
+#pragma unroll
+        for (int u = 0; u < kU; ++u) {
+          const int64_t rr = r + u * stride;
+          ok[u] = rr < num_rows && (mask == nullptr || mask[rr] != 0);
+          if (ok[u]) v[u].load(x + rr * ldx + c0);
+        }
+#pragma unroll
+        for (int u = 0; u < kU; ++u) {
+          if (!ok[u]) continue;
+          float f[VEC];
+          v[u].unpack(f);
+#pragma unroll
+          for (int k = 0; k < VEC; ++k) {
+            const double d = double(f[k]) - p[k];   // exact for fp32 values less than 2^29 apart in scale
+            s[k] += d;
+            q[k] = fma(d, d, q[k]);
+          }
+        }
+      }
+    }
+  } else if (cvalid) {
     // kU row loads in flight per thread (latency, not issue, bounds a one-load loop); fp32 partials
     // over those rows, flushed into the fp64 accumulators: error of a partial <= kU ulp(fp32)
     const int64_t stride = int64_t(gridDim.y) * rpc;
@@ -156,10 +194,14 @@ __global__ void __launch_bounds__(kCta) colstats_kernel(const T* __restrict__ x,
 // 32 channels x 8 row-block ranges per CTA: group g sums the partials y in [g*span, (g+1)*span) in order (eight
 // independent loads ahead of the adds), the eight range sums are combined in group order: a fixed summation tree
 // (deterministic) whose serial chain is row_blocks / 8 long (one thread per channel walking all ~1000 partials made
-// this tiny kernel cost as much as the statistics pass on L2-resident graphs)
+// this tiny kernel cost as much as the statistics pass on L2-resident graphs).  With a pivot p (colstats of fp32
+// rows) the sums are of d = x - p over num_rows rows and are turned back into sums of x and x^2 here; for a
+// constant column (d == 0) that leaves out0 = N p exactly and out1 = fl(N p * p).
 constexpr int kFinalGroups = 8;
 __global__ void __launch_bounds__(32 * kFinalGroups) colstats_final_kernel(const double* __restrict__ partial,
                                                                            int row_blocks, int64_t C,
+                                                                           const float* __restrict__ pivot,
+                                                                           int64_t num_rows,
                                                                            double* __restrict__ out0,
                                                                            double* __restrict__ out1) {
   __shared__ double sh[2][kFinalGroups][32];
@@ -192,6 +234,11 @@ __global__ void __launch_bounds__(32 * kFinalGroups) colstats_final_kernel(const
     double ta = 0.0, tb = 0.0;
 #pragma unroll
     for (int k = 0; k < kFinalGroups; ++k) { ta += sh[0][k][cx]; tb += sh[1][k][cx]; }
+    if (pivot) {
+      const double p = pivot[c], np = double(num_rows) * p;
+      tb = (tb + 2.0 * p * ta) + np * p;
+      ta = ta + np;
+    }
     if (out0) out0[c] = ta;
     if (out1) out1[c] = tb;
   }
@@ -206,7 +253,8 @@ __global__ void graphnorm_prepare_kernel(const double* __restrict__ colsum, cons
   const double n = double(num_rows);
   const double mu = colsum[c] / n;
   const double a = double(mean_scale[c]);
-  double var = colsq[c] / n - mu * mu * (2.0 * a - a * a);
+  // sum x^2 - fl(sum x * mu): exactly 0 for a constant column whose sums colstats formed about a pivot
+  double var = (colsq[c] - __dmul_rn(colsum[c], mu) * (2.0 * a - a * a)) / n;
   if (var < 0.0) var = 0.0;
   mean_out[c] = float(mu);
   rstd_out[c] = float(1.0 / sqrt(var + double(eps)));
@@ -509,16 +557,20 @@ static int colstats_impl(const void* x, int dtype, int64_t N, int64_t C, int64_t
   GMLM_REQUIRE(ws && ws_bytes >= partial_bytes(C), "colstats: workspace too small");
   double* partial = static_cast<double*>(ws);
   const bool v = vec_ok(dtype, C, {x}, {ldx});
+  // fp32 sums are taken about the first row (a row mask would leave the pivoted row count unknown)
+  const float* pivot = dtype == GMLM_F32 && N > 0 && mask == nullptr ? static_cast<const float*>(x) : nullptr;
   int row_blocks = 1;
   int rc = dispatch(dtype, v, [&]<typename T, int VEC>() -> int {
     Tile t = make_tile(N, C, VEC, resident_ctas<colstats_kernel<T, VEC>>());
     row_blocks = int(t.grid.y);
-    colstats_kernel<T, VEC><<<t.grid, kCta, 0, st>>>(static_cast<const T*>(x), N, C, ldx, mask, t.tpr, partial);
+    colstats_kernel<T, VEC><<<t.grid, kCta, 0, st>>>(static_cast<const T*>(x), N, C, ldx, mask, pivot, t.tpr,
+                                                     partial);
     GMLM_LAUNCH_CHECK();
     return GMLM_OK;
   });
   if (rc) return rc;
-  colstats_final_kernel<<<unsigned((C + 31) / 32), 32 * kFinalGroups, 0, st>>>(partial, row_blocks, C, out0, out1);
+  colstats_final_kernel<<<unsigned((C + 31) / 32), 32 * kFinalGroups, 0, st>>>(partial, row_blocks, C, pivot, N,
+                                                                               out0, out1);
   GMLM_LAUNCH_CHECK();
   return GMLM_OK;
 }
@@ -574,7 +626,8 @@ int gmlm_graphnorm_bwd_stats(const void* x, const void* gy, int dtype, int64_t N
     return GMLM_OK;
   });
   if (rc) return rc;
-  colstats_final_kernel<<<unsigned((C + 31) / 32), 32 * kFinalGroups, 0, st>>>(partial, row_blocks, C, sum_g, sum_go);
+  colstats_final_kernel<<<unsigned((C + 31) / 32), 32 * kFinalGroups, 0, st>>>(partial, row_blocks, C, nullptr, N,
+                                                                               sum_g, sum_go);
   GMLM_LAUNCH_CHECK();
   return GMLM_OK;
 }

@@ -239,16 +239,28 @@ def _graphnorm_bwd(x, gy, mean, rstd, weight, bias, mean_scale, fuse_gelu, need_
 
 # ------------------------------------------------------------------------------ A13 LayerNorm
 def layer_norm_ok(x: torch.Tensor) -> bool:
-    """Shapes the row-wise kernel takes: CUDA fp32/bf16 [N, C], C a multiple of the 16-byte pack, C <= 1024."""
+    """Shapes the row-wise kernel takes: CUDA fp32/bf16 [N, C], C a multiple of the 16-byte pack, C <= 1024.
+    Any strides and storage offset: a view the kernel cannot read in 16-byte packs is copied first."""
     if not (x.is_cuda and x.dim() == 2 and x.dtype in _DT and x.size(0) >= 1):
         return False
     vec = 4 if x.dtype == torch.float32 else 8
     return x.size(1) % vec == 0 and 0 < x.size(1) <= _lib.load().gmlm_layernorm_max_channels(_DT[x.dtype])
 
 
+def _packed_rows(t: torch.Tensor) -> torch.Tensor:
+    """``_rowmajor`` plus what the LayerNorm kernel reads in 16-byte packs: a 16-byte aligned base and a leading
+    dimension that is a whole number of packs.  A view that lacks either (a column slice at an odd offset, the
+    gradient autograd hands back for one block of a ``torch.cat``) is copied."""
+    t = _rowmajor(t)
+    vec = 16 // t.element_size()
+    if t.data_ptr() % 16 or _ld(t) % vec:
+        t = t.clone(memory_format=torch.contiguous_format)
+    return t
+
+
 def _layernorm_fwd(x, weight, bias, eps):
     lib = _lib.load()
-    x = _rowmajor(x)
+    x = _packed_rows(x)
     n, c = x.shape
     dev = x.device
     weight, bias = _f32c(weight), _f32c(bias)
@@ -264,10 +276,10 @@ def _layernorm_fwd(x, weight, bias, eps):
 
 def _layernorm_bwd(x, gy, mean, rstd, weight, need_gx):
     lib = _lib.load()
-    x = _rowmajor(x)
-    gy = _rowmajor(gy)
+    x = _packed_rows(x)
     if gy.dtype != x.dtype:
         gy = gy.to(x.dtype)
+    gy = _packed_rows(gy)
     n, c = x.shape
     dev = x.device
     weight = _f32c(weight)
