@@ -21,8 +21,15 @@
 // Attention dropout (upstream: F.dropout on alpha): keep[e,h] comes from a counter-based hash of (seed, CSR
 // position, head), so forward, backward and `gmlm_gat_dropout_mask` (tests) agree without storing a mask.
 //
-// Lane mapping: one warp per row / chunk; lane owns packs p = lane, lane+32, ... of the H*C features (a pack never
-// straddles heads: C % VEC == 0), at most CH packs per lane.
+// Lane mapping: one warp per row / chunk and head group; lane owns packs p = lane, lane+32, ... of the group's
+// features (a pack never straddles heads: C % VEC == 0), at most CH packs per lane.
+//
+// Head groups: the heads of a row are independent in the softmax, so a row wider than one warp's CH packs is cut
+// into groups of whole heads (GatParams::hg heads each), one per grid.y index, each walking the same CSR row or hub
+// chunk.  A group reads and writes only its own heads; a_src, a_dst, m, l and the dropout hash keep the global head
+// index and H as the stride, so the result does not depend on the cut.  Rows that fit one warp are one group
+// (grid.y = 1, hg = H) and run the G = false instantiations, whose code has no group offsets at all; grouped rows run
+// G = true at the widest CH of their path.
 #include "common.cuh"
 
 namespace gmlm {
@@ -52,29 +59,37 @@ struct GatParams {
   const float* a_src;   // [num_src, H]
   const float* a_dst;   // [num_rows, H]
   int H, C;
+  int hg;               // heads per group (grid.y = ceil(H / hg)); hg = H: the whole row in one group
   float slope, p_drop;
   uint64_t seed;
   int32_t hub_thresh;
 };
 
-template <typename T, int VEC, int CH>
+template <typename T, int VEC, int CH, bool G>
 struct Lane {
   int head[CH];
   bool valid[CH];
   int64_t f[CH];
-  __device__ __forceinline__ void init(int lane, int H, int C) {
+  // features [h0*C, h1*C) of head group blockIdx.y (G), or all H*C features
+  __device__ __forceinline__ void init(int lane, const GatParams& p) {
+    int64_t f0 = 0, f1 = int64_t(p.H) * p.C;
+    if constexpr (G) {
+      const int h0 = int(blockIdx.y) * p.hg, h1 = min(h0 + p.hg, p.H);
+      f0 = int64_t(h0) * p.C;
+      f1 = int64_t(h1) * p.C;
+    }
 #pragma unroll
     for (int ch = 0; ch < CH; ++ch) {
-      f[ch] = int64_t(ch * 32 + lane) * VEC;
-      valid[ch] = f[ch] < int64_t(H) * C;
-      head[ch] = valid[ch] ? int(f[ch] / C) : 0;
+      f[ch] = f0 + int64_t(ch * 32 + lane) * VEC;
+      valid[ch] = f[ch] < f1;
+      head[ch] = valid[ch] ? int(f[ch] / p.C) : 0;
     }
   }
 };
 
 // online-softmax scan of edges [b, e) of destination row `row`
-template <typename T, int VEC, int CH>
-__device__ __forceinline__ void gat_scan(const GatParams& p, const Lane<T, VEC, CH>& ln, int64_t row, int32_t b, int32_t e,
+template <typename T, int VEC, int CH, bool G>
+__device__ __forceinline__ void gat_scan(const GatParams& p, const Lane<T, VEC, CH, G>& ln, int64_t row, int32_t b, int32_t e,
                                          float (&m)[CH], float (&l)[CH], float (&acc)[CH][VEC]) {
   const T* __restrict__ z = static_cast<const T*>(p.z);
   float ad[CH];
@@ -124,7 +139,7 @@ __device__ __forceinline__ void gat_scan(const GatParams& p, const Lane<T, VEC, 
   }
 }
 
-template <typename T, int VEC, int CH>
+template <typename T, int VEC, int CH, bool G>
 __global__ void __launch_bounds__(256) gat_rows_kernel(const GatParams p, int64_t num_rows, T* __restrict__ out,
                                                        int64_t ldo, float* __restrict__ m_out, float* __restrict__ l_out) {
   const int64_t r = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
@@ -132,10 +147,10 @@ __global__ void __launch_bounds__(256) gat_rows_kernel(const GatParams p, int64_
   if (r >= num_rows) return;
   const int32_t b = __ldg(p.rowptr + r), e = __ldg(p.rowptr + r + 1);
   if (e - b > p.hub_thresh) return;                 // a hub row: chunk kernel + final kernel
-  Lane<T, VEC, CH> ln;
-  ln.init(lane, p.H, p.C);
+  Lane<T, VEC, CH, G> ln;
+  ln.init(lane, p);
   float m[CH], l[CH], acc[CH][VEC];
-  gat_scan<T, VEC, CH>(p, ln, r, b, e, m, l, acc);
+  gat_scan<T, VEC, CH, G>(p, ln, r, b, e, m, l, acc);
   const float keep_scale = p.p_drop > 0.f ? 1.0f / (1.0f - p.p_drop) : 1.0f;
 #pragma unroll
   for (int ch = 0; ch < CH; ++ch) {
@@ -154,7 +169,7 @@ __global__ void __launch_bounds__(256) gat_rows_kernel(const GatParams p, int64_
   }
 }
 
-template <typename T, int VEC, int CH>
+template <typename T, int VEC, int CH, bool G>
 __global__ void __launch_bounds__(256) gat_chunk_kernel(const GatParams p, const int32_t* __restrict__ chunk_beg,
                                                         const int32_t* __restrict__ chunk_end,
                                                         const int32_t* __restrict__ chunk_row, int64_t n_chunks,
@@ -163,10 +178,10 @@ __global__ void __launch_bounds__(256) gat_chunk_kernel(const GatParams p, const
   const int64_t c = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (c >= n_chunks) return;
-  Lane<T, VEC, CH> ln;
-  ln.init(lane, p.H, p.C);
+  Lane<T, VEC, CH, G> ln;
+  ln.init(lane, p);
   float m[CH], l[CH], acc[CH][VEC];
-  gat_scan<T, VEC, CH>(p, ln, __ldg(chunk_row + c), __ldg(chunk_beg + c), __ldg(chunk_end + c), m, l, acc);
+  gat_scan<T, VEC, CH, G>(p, ln, __ldg(chunk_row + c), __ldg(chunk_beg + c), __ldg(chunk_end + c), m, l, acc);
   const int64_t hc = int64_t(p.H) * p.C;
 #pragma unroll
   for (int ch = 0; ch < CH; ++ch) {
@@ -217,8 +232,8 @@ __global__ void chunk_rows_kernel(const int32_t* __restrict__ hub_row, const int
 
 // ---------------------------------------------------------------------------------- backward, edge pass
 // one warp per (row | chunk): alpha_eff[k,h], d_score[k,h] for its edges, partial da_dst[., h]
-template <typename T, int VEC, int CH>
-__device__ __forceinline__ void gat_bwd_scan(const GatParams& p, const Lane<T, VEC, CH>& ln, int lane, int64_t row,
+template <typename T, int VEC, int CH, bool G>
+__device__ __forceinline__ void gat_bwd_scan(const GatParams& p, const Lane<T, VEC, CH, G>& ln, int lane, int64_t row,
                                              int32_t b, int32_t e, const T* __restrict__ g, int64_t ldg,
                                              const float* __restrict__ m_in, const float* __restrict__ l_in,
                                              const float* __restrict__ t_in, float* __restrict__ alpha_eff,
@@ -233,8 +248,13 @@ __device__ __forceinline__ void gat_bwd_scan(const GatParams& p, const Lane<T, V
       pk.unpack(gf[ch]);
     }
   }
-  // lane h (< H) carries the per-head scalars of head h
-  const int hh = lane < p.H ? lane : 0;
+  // lane j (< the group's head count) carries the per-head scalars of head h0 + j
+  int h0 = 0, nh = p.H;
+  if constexpr (G) {
+    h0 = int(blockIdx.y) * p.hg;
+    nh = min(p.hg, p.H - h0);
+  }
+  const int hh = h0 + (lane < nh ? lane : 0);
   const float ad = __ldg(p.a_dst + row * p.H + hh), mm = __ldg(m_in + row * p.H + hh);
   const float inv_l = 1.0f / (__ldg(l_in + row * p.H + hh) + 1e-16f), tt = __ldg(t_in + row * p.H + hh);
   const float keep_scale = p.p_drop > 0.f ? 1.0f / (1.0f - p.p_drop) : 1.0f;
@@ -253,30 +273,31 @@ __device__ __forceinline__ void gat_bwd_scan(const GatParams& p, const Lane<T, V
 #pragma unroll
       for (int v = 0; v < VEC; ++v) part[ch] = fmaf(gf[ch][v], zf[v], part[ch]);
     }
-    float dot_mine = 0.f;                              // <g[row,h,:], z[s,h,:]> for h = lane
-    for (int h = 0; h < p.H; ++h) {
+    float dot_mine = 0.f;                              // <g[row,h,:], z[s,h,:]> for h = h0 + lane
+    for (int j = 0; j < nh; ++j) {
       float v = 0.f;
 #pragma unroll
-      for (int ch = 0; ch < CH; ++ch) v += (ln.valid[ch] && ln.head[ch] == h) ? part[ch] : 0.f;
+      for (int ch = 0; ch < CH; ++ch) v += (ln.valid[ch] && ln.head[ch] == h0 + j) ? part[ch] : 0.f;
       v = warp_sum(v);
-      if (lane == h) dot_mine = v;
+      if (lane == j) dot_mine = v;
     }
-    if (lane < p.H) {
-      const float raw = __ldg(p.a_src + int64_t(s) * p.H + lane) + ad;
+    if (lane < nh) {
+      const int hd = G ? hh : lane;                    // this lane's head (global index)
+      const float raw = __ldg(p.a_src + int64_t(s) * p.H + hd) + ad;
       const float alpha = expf(lrelu(raw, p.slope) - mm) * inv_l;
-      const bool keep = p.p_drop <= 0.f || drop_keep(p.seed, uint64_t(k) * p.H + lane, p.p_drop);
+      const bool keep = p.p_drop <= 0.f || drop_keep(p.seed, uint64_t(k) * p.H + hd, p.p_drop);
       const float ks = keep ? keep_scale : 0.f;
       const float de = alpha * (ks * dot_mine - tt);
       const float ds = raw > 0.f ? de : de * p.slope;
-      alpha_eff[int64_t(k) * p.H + lane] = alpha * ks;
-      d_score[int64_t(k) * p.H + lane] = ds;
+      alpha_eff[int64_t(k) * p.H + hd] = alpha * ks;
+      d_score[int64_t(k) * p.H + hd] = ds;
       dsum += ds;
     }
   }
-  if (lane < p.H) da_dst_out[lane] = dsum;
+  if (lane < nh) da_dst_out[G ? hh : lane] = dsum;
 }
 
-template <typename T, int VEC, int CH>
+template <typename T, int VEC, int CH, bool G>
 __global__ void __launch_bounds__(256) gat_bwd_rows_kernel(const GatParams p, int64_t num_rows, const T* __restrict__ g,
                                                            int64_t ldg, const float* __restrict__ m_in,
                                                            const float* __restrict__ l_in, const float* __restrict__ t_in,
@@ -287,12 +308,12 @@ __global__ void __launch_bounds__(256) gat_bwd_rows_kernel(const GatParams p, in
   if (r >= num_rows) return;
   const int32_t b = __ldg(p.rowptr + r), e = __ldg(p.rowptr + r + 1);
   if (e - b > p.hub_thresh) return;
-  Lane<T, VEC, CH> ln;
-  ln.init(lane, p.H, p.C);
-  gat_bwd_scan<T, VEC, CH>(p, ln, lane, r, b, e, g, ldg, m_in, l_in, t_in, alpha_eff, d_score, da_dst + r * p.H);
+  Lane<T, VEC, CH, G> ln;
+  ln.init(lane, p);
+  gat_bwd_scan<T, VEC, CH, G>(p, ln, lane, r, b, e, g, ldg, m_in, l_in, t_in, alpha_eff, d_score, da_dst + r * p.H);
 }
 
-template <typename T, int VEC, int CH>
+template <typename T, int VEC, int CH, bool G>
 __global__ void __launch_bounds__(256) gat_bwd_chunk_kernel(const GatParams p, const int32_t* __restrict__ chunk_beg,
                                                             const int32_t* __restrict__ chunk_end,
                                                             const int32_t* __restrict__ chunk_row, int64_t n_chunks,
@@ -303,9 +324,9 @@ __global__ void __launch_bounds__(256) gat_bwd_chunk_kernel(const GatParams p, c
   const int64_t c = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (c >= n_chunks) return;
-  Lane<T, VEC, CH> ln;
-  ln.init(lane, p.H, p.C);
-  gat_bwd_scan<T, VEC, CH>(p, ln, lane, __ldg(chunk_row + c), __ldg(chunk_beg + c), __ldg(chunk_end + c), g, ldg, m_in,
+  Lane<T, VEC, CH, G> ln;
+  ln.init(lane, p);
+  gat_bwd_scan<T, VEC, CH, G>(p, ln, lane, __ldg(chunk_row + c), __ldg(chunk_beg + c), __ldg(chunk_end + c), g, ldg, m_in,
                            l_in, t_in, alpha_eff, d_score, da_part + c * p.H);
 }
 
@@ -356,7 +377,37 @@ int dispatch_geo(int dtype, int64_t hc, bool aligned, Fn&& fn) {
   return fail(GMLM_ERR_INVALID, "gat: heads * head_dim = %lld is wider than this kernel covers", (long long)hc);
 }
 
+// a row that fits one warp: the instantiation for its width, no group offsets (G = false); a row cut into head groups:
+// the widest instantiation of its path (G = true)
+template <typename Fn>
+int dispatch_gat(int dtype, int64_t hc, bool aligned, int n_groups, Fn&& fn) {
+  if (n_groups == 1)
+    return dispatch_geo(dtype, hc, aligned, [&]<typename T, int VEC, int CH>() -> int {
+      return fn.template operator()<T, VEC, CH, false>();
+    });
+  if (dtype == GMLM_F32) return aligned ? fn.template operator()<float, 4, 8, true>() : fn.template operator()<float, 1, 8, true>();
+  return aligned ? fn.template operator()<__nv_bfloat16, 8, 4, true>() : fn.template operator()<__nv_bfloat16, 1, 8, true>();
+}
+
 inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+
+// The head-group cut of a row: the fewest groups of whole heads whose width fits the widest instantiation of the
+// path (1024 features on 16-byte packs, 256 on scalar packs), heads spread evenly over the groups.  A row that fits
+// is one group of all H heads.
+struct HeadGroups {
+  int hg, n;
+};
+inline int head_groups(int heads, int head_dim, bool aligned, const char* who, HeadGroups* out) {
+  const int64_t cap = aligned ? 1024 : 256;
+  if (head_dim > cap)
+    return fail(GMLM_ERR_INVALID, "%s: one head of head_dim = %d is wider than this kernel covers (%lld features%s)",
+                who, head_dim, (long long)cap, aligned ? "" : " on the scalar path: odd or misaligned widths");
+  const int per = int(cap / head_dim);               // most heads one group can take
+  const int n = (heads + per - 1) / per;
+  out->n = n;
+  out->hg = (heads + n - 1) / n;
+  return GMLM_OK;
+}
 
 }  // namespace
 }  // namespace gmlm
@@ -364,7 +415,8 @@ inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) 
 using namespace gmlm;
 
 extern "C" size_t gmlm_gat_workspace_bytes(int64_t n_chunks, int heads, int head_dim) {
-  // chunk_row (i32) + pm, pl (f32 [chunks, H]) + pacc (f32 [chunks, H*C])
+  // chunk_row (i32) + pm, pl (f32 [chunks, H]) + pacc (f32 [chunks, H*C]); the head groups of a chunk write
+  // disjoint heads / features of the same arrays, so the split needs no more
   return size_t(n_chunks) * (4 + size_t(heads) * 8 + size_t(heads) * head_dim * 4) + 1024;
 }
 
@@ -386,23 +438,25 @@ extern "C" int gmlm_gat_fused_fwd(const int32_t* rowptr, const int32_t* col, int
                "gat_fused_fwd: hub plan / workspace missing");
   const int v = dtype == GMLM_F32 ? 4 : 8;
   const bool aligned = head_dim % v == 0 && ldz % v == 0 && ldo % v == 0 && al16(z) && al16(out);
+  HeadGroups hgp;
+  if (int rc = head_groups(heads, head_dim, aligned, "gat_fused_fwd", &hgp)) return rc;
   cudaStream_t st = as_stream(stream);
-  GatParams p{rowptr, col, z, ldz, a_src, a_dst, heads, head_dim, negative_slope, p_drop, seed,
+  GatParams p{rowptr, col, z, ldz, a_src, a_dst, heads, head_dim, hgp.hg, negative_slope, p_drop, seed,
               n_hub > 0 ? hub_thresh : 0x7fffffff};
   Carver cv(ws);
   int32_t* chunk_row = n_hub ? cv.take<int32_t>(n_chunks) : nullptr;
   float* pm = n_hub ? cv.take<float>(n_chunks * heads) : nullptr;
   float* pl = n_hub ? cv.take<float>(n_chunks * heads) : nullptr;
   float* pacc = n_hub ? cv.take<float>(n_chunks * hc) : nullptr;
-  const unsigned blocks = unsigned((num_rows * 32 + 255) / 256);
-  int rc = dispatch_geo(dtype, hc, aligned, [&]<typename T, int VEC, int CH>() -> int {
-    gat_rows_kernel<T, VEC, CH><<<blocks, 256, 0, st>>>(p, num_rows, static_cast<T*>(out), ldo, m_out, l_out);
+  const dim3 grid(unsigned((num_rows * 32 + 255) / 256), unsigned(hgp.n));
+  const dim3 cgrid(unsigned((n_chunks * 32 + 255) / 256), unsigned(hgp.n));
+  int rc = dispatch_gat(dtype, hc, aligned, hgp.n, [&]<typename T, int VEC, int CH, bool G>() -> int {
+    gat_rows_kernel<T, VEC, CH, G><<<grid, 256, 0, st>>>(p, num_rows, static_cast<T*>(out), ldo, m_out, l_out);
     GMLM_LAUNCH_CHECK();
     if (n_hub) {
       chunk_rows_kernel<<<unsigned(n_hub), 128, 0, st>>>(hub_row, hub_chunk_ptr, n_hub, chunk_row);
       GMLM_LAUNCH_CHECK();
-      gat_chunk_kernel<T, VEC, CH><<<unsigned((n_chunks * 32 + 255) / 256), 256, 0, st>>>(p, chunk_beg, chunk_end,
-                                                                                          chunk_row, n_chunks, pm, pl, pacc);
+      gat_chunk_kernel<T, VEC, CH, G><<<cgrid, 256, 0, st>>>(p, chunk_beg, chunk_end, chunk_row, n_chunks, pm, pl, pacc);
       GMLM_LAUNCH_CHECK();
       gat_final_kernel<T><<<unsigned(n_hub), 256, 0, st>>>(hub_row, hub_chunk_ptr, n_hub, heads, head_dim, p_drop, pm, pl,
                                                            pacc, static_cast<T*>(out), ldo, m_out, l_out);
@@ -432,21 +486,24 @@ extern "C" int gmlm_gat_bwd_edges(const int32_t* rowptr, const int32_t* col, int
                "gat_bwd_edges: hub plan / workspace missing");
   const int v = dtype == GMLM_F32 ? 4 : 8;
   const bool aligned = head_dim % v == 0 && ldz % v == 0 && ldg % v == 0 && al16(z) && al16(g);
+  HeadGroups hgp;
+  if (int rc = head_groups(heads, head_dim, aligned, "gat_bwd_edges", &hgp)) return rc;
   cudaStream_t st = as_stream(stream);
-  GatParams p{rowptr, col, z, ldz, a_src, a_dst, heads, head_dim, negative_slope, p_drop, seed,
+  GatParams p{rowptr, col, z, ldz, a_src, a_dst, heads, head_dim, hgp.hg, negative_slope, p_drop, seed,
               n_hub > 0 ? hub_thresh : 0x7fffffff};
   Carver cv(ws);
   int32_t* chunk_row = n_hub ? cv.take<int32_t>(n_chunks) : nullptr;
   float* da_part = n_hub ? cv.take<float>(n_chunks * heads) : nullptr;
-  const unsigned blocks = unsigned((num_rows * 32 + 255) / 256);
-  return dispatch_geo(dtype, hc, aligned, [&]<typename T, int VEC, int CH>() -> int {
-    gat_bwd_rows_kernel<T, VEC, CH><<<blocks, 256, 0, st>>>(p, num_rows, static_cast<const T*>(g), ldg, m_in, l_in, t_in,
+  const dim3 grid(unsigned((num_rows * 32 + 255) / 256), unsigned(hgp.n));
+  const dim3 cgrid(unsigned((n_chunks * 32 + 255) / 256), unsigned(hgp.n));
+  return dispatch_gat(dtype, hc, aligned, hgp.n, [&]<typename T, int VEC, int CH, bool G>() -> int {
+    gat_bwd_rows_kernel<T, VEC, CH, G><<<grid, 256, 0, st>>>(p, num_rows, static_cast<const T*>(g), ldg, m_in, l_in, t_in,
                                                             alpha_eff, d_score, da_dst);
     GMLM_LAUNCH_CHECK();
     if (n_hub) {
       chunk_rows_kernel<<<unsigned(n_hub), 128, 0, st>>>(hub_row, hub_chunk_ptr, n_hub, chunk_row);
       GMLM_LAUNCH_CHECK();
-      gat_bwd_chunk_kernel<T, VEC, CH><<<unsigned((n_chunks * 32 + 255) / 256), 256, 0, st>>>(
+      gat_bwd_chunk_kernel<T, VEC, CH, G><<<cgrid, 256, 0, st>>>(
           p, chunk_beg, chunk_end, chunk_row, n_chunks, static_cast<const T*>(g), ldg, m_in, l_in, t_in, alpha_eff,
           d_score, da_part);
       GMLM_LAUNCH_CHECK();

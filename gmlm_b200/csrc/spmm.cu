@@ -854,7 +854,10 @@ template <typename T, int VEC>
 int launch_vec(Job& job, cudaStream_t st) {
   const int64_t width = job.rows.slab_width ? job.rows.slab_width : job.rows.feat;
   const int64_t nvec = (width + VEC - 1) / VEC;
-  if (job.rows.slab_width) GMLM_REQUIRE(nvec <= 128, "spmm: per-head width above 128 packs is not supported");
+  if (job.rows.slab_width) GMLM_REQUIRE(nvec <= 256, "spmm: per-head width above 256 packs is not supported");
+  // one head slab per warp up to 256 packs: the GAT input gradient of heads wider than 128 packs (520 fp32 features on
+  // 16-byte packs, 130 on scalar packs); every other width keeps the instantiations below
+  if (job.rows.slab_width && nvec > 128) return launch_geo<T, VEC, 8, 32, 1, 1>(job, st);
   // narrow rows without head slabs: the warp-uniform edge walk (spmm_variant 2 keeps the general kernel for A/B)
   const bool narrow = job.do_rows && job.rows.slab_stride == 0 && job.rows.w_stride <= 1 && !job.rows.single &&
                       tuning_spmm_variant() != 2;

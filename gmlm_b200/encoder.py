@@ -12,6 +12,11 @@ What changes relative to the reference body (results stay within the parity tole
     discarded by the reference, so ``residual_proj3`` gets no gradient there either;
   * activation checkpointing (main.py:278) stays available (``use_checkpoint=True``) and is
     re-entrant-safe: the ops use no RNG and the graph cache is read-only.
+
+``conv="gat"`` builds the same body on GAT edge-softmax layers (BASELINE configs[2]): ``gat1..gat4`` =
+``GATConv(dims[k], dims[k+1] // heads, heads)`` with concatenated heads and attention dropout 0 in place of
+``rgcn1..rgcn4``; every other submodule keeps its name and code.  The four layers share one self-looped CSR
+(``get_loop_graph``); no edge types are computed.  fp32 activations only (eval mode, or autocast with fp32 results).
 """
 from __future__ import annotations
 
@@ -24,6 +29,7 @@ import torch.nn.functional as F
 from torch.utils.checkpoint import checkpoint
 
 from .graph import _LOCK, _tensor_key, get_rel_graph
+from .attn import GATConv, get_loop_graph
 from .nn import GraphNorm, RGCNConv
 from .ops import edge_type_from_degree, layer_norm, layer_norm_ok, linear_nt, soft_masking_gnn_input
 
@@ -97,16 +103,28 @@ def cached_edge_type(edge_index: torch.Tensor, num_nodes: int) -> torch.Tensor:
 class GraphEncoder(nn.Module):
     def __init__(self, gnn_in_channels: int, hidden_channels: int, out_dim: int, num_relations: int = 5,
                  num_bases: int = 30, dropout_rate: float = 0.3, use_checkpoint: bool = False,
-                 act_dtype: Optional[torch.dtype] = None):
+                 act_dtype: Optional[torch.dtype] = None, conv: str = "rgcn", heads: int = 8):
         super().__init__()
         h = hidden_channels
         dims = [gnn_in_channels, h, 2 * h, 4 * h, 8 * h]
+        if conv not in ("rgcn", "gat"):
+            raise ValueError(f"GraphEncoder: conv must be 'rgcn' or 'gat', got {conv!r}")
+        if conv == "gat":
+            if heads < 1 or any(d % heads for d in dims[1:]):
+                raise ValueError(f"GraphEncoder: heads = {heads} must divide every GAT layer width {dims[1:]}")
+            if act_dtype == torch.bfloat16:
+                raise NotImplementedError("GraphEncoder: the GAT encoder runs fp32 activations (eval or autocast), "
+                                          "not the bf16 pipeline")
         self.dims = dims
+        self.conv = conv
         self.gnn_mask_token_embed = nn.Parameter(torch.zeros(1, gnn_in_channels))   # main.py:185-186
         nn.init.xavier_uniform_(self.gnn_mask_token_embed)
         for k in range(4):                                                          # main.py:189-203
-            setattr(self, f"rgcn{k+1}", RGCNConv(dims[k], dims[k + 1], num_relations=num_relations,
-                                                 num_bases=num_bases, out_dtype=act_dtype))
+            if conv == "gat":
+                setattr(self, f"gat{k+1}", GATConv(dims[k], dims[k + 1] // heads, heads=heads))
+            else:
+                setattr(self, f"rgcn{k+1}", RGCNConv(dims[k], dims[k + 1], num_relations=num_relations,
+                                                     num_bases=num_bases, out_dtype=act_dtype))
             setattr(self, f"gnorm{k+1}", GraphNorm(dims[k + 1]))
             setattr(self, f"dropout{k+1}", nn.Dropout(dropout_rate))
         self.residual_proj1 = nn.Linear(gnn_in_channels, h)                         # main.py:205-207
@@ -117,7 +135,7 @@ class GraphEncoder(nn.Module):
         self.use_checkpoint = use_checkpoint
 
     def _block(self, k: int):
-        conv, norm, drop = getattr(self, f"rgcn{k}"), getattr(self, f"gnorm{k}"), getattr(self, f"dropout{k}")
+        conv, norm, drop = getattr(self, f"{self.conv}{k}"), getattr(self, f"gnorm{k}"), getattr(self, f"dropout{k}")
 
         def run(x, graph):
             y = conv(x, graph)
@@ -147,9 +165,12 @@ class GraphEncoder(nn.Module):
     def get_graph_embeddings(self, x_feat: torch.Tensor, edge_index: torch.Tensor,
                              edge_type: Optional[torch.Tensor] = None, return_layers: bool = False):
         n = x_feat.size(0)
-        if edge_type is None:
-            edge_type = cached_edge_type(edge_index, n)
-        graph = get_rel_graph(edge_index, edge_type, n, self.num_relations)
+        if self.conv == "gat":
+            graph = get_loop_graph(edge_index, n)     # edge_type is not used by GAT layers
+        else:
+            if edge_type is None:
+                edge_type = cached_edge_type(edge_index, n)
+            graph = get_rel_graph(edge_index, edge_type, n, self.num_relations)
         outs = []
         x1 = self._run(1, x_feat, graph)
         outs.append(x1)                              # pre-residual outputs feed the fusion (main.py:279)

@@ -31,7 +31,9 @@ class GraphedEncoderStep:
         self.autocast = bool(autocast)
         n = x.size(0)
         self.edge_index = edge_index
-        self.edge_type = edge_type if edge_type is not None else cached_edge_type(edge_index, n)
+        if edge_type is None and getattr(encoder, "conv", "rgcn") == "rgcn":
+            edge_type = cached_edge_type(edge_index, n)           # GAT layers take no edge types
+        self.edge_type = edge_type
         self.static_x = x.detach().clone().requires_grad_(x_requires_grad)
         side = torch.cuda.Stream(device=x.device)
         side.wait_stream(torch.cuda.current_stream(x.device))
