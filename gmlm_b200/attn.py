@@ -77,9 +77,10 @@ def get_loop_graph(edge_index: torch.Tensor, num_nodes: int) -> LoopGraph:
 
 
 def _with_w(csr: CSR, w: torch.Tensor) -> CSR:
-    """A shallow view of ``csr`` carrying different per-edge weights."""
+    """A shallow view of ``csr`` carrying different per-edge weights (its band plan's hub_w no longer applies)."""
     c = CSR(**{k: getattr(csr, k) for k in csr.__dataclass_fields__})
     c.w = w
+    c.hub_w = None
     return c
 
 

@@ -289,6 +289,93 @@ __global__ void hub_fill_chunks_kernel(const int32_t* __restrict__ rowptr, const
   }
 }
 
+// ------------------------------------------------------------------ band-ordered hub plan
+// The hub edges listed row by row (hub_off[h] = first position of hub row h): key = gathered row, value = position.
+__global__ void hub_band_keys_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
+                                     const int32_t* __restrict__ hub_row, const int32_t* __restrict__ hub_off,
+                                     int64_t n_hub, uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
+  const int64_t h = (blockIdx.x * int64_t(blockDim.x) + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (h >= n_hub) return;
+  const int32_t e0 = rowptr[hub_row[h]], o0 = hub_off[h], n = hub_off[h + 1] - o0;
+  for (int32_t j = lane; j < n; j += 32) {
+    keys[o0 + j] = uint32_t(col[e0 + j]);
+    vals[o0 + j] = o0 + j;
+  }
+}
+
+// key = hub row of list position vals[k] (last h with hub_off[h] <= vals[k])
+__global__ void hub_band_rowkey_kernel(const int32_t* __restrict__ vals, int64_t n, const int32_t* __restrict__ hub_off,
+                                       int64_t n_hub, uint32_t* __restrict__ keys) {
+  for (int64_t k = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; k < n; k += int64_t(gridDim.x) * blockDim.x) {
+    const int32_t i = vals[k];
+    int64_t lo = 0, hi = n_hub;
+    while (hi - lo > 1) {
+      const int64_t mid = (lo + hi) >> 1;
+      if (hub_off[mid] <= i) lo = mid; else hi = mid;
+    }
+    keys[k] = uint32_t(lo);
+  }
+}
+
+__global__ void hub_band_gather_kernel(const uint32_t* __restrict__ row_key, const int32_t* __restrict__ vals, int64_t n,
+                                       const int32_t* __restrict__ rowptr, const int32_t* __restrict__ hub_row,
+                                       const int32_t* __restrict__ hub_off, const int32_t* __restrict__ col,
+                                       const float* __restrict__ w, int32_t* __restrict__ hub_col,
+                                       float* __restrict__ hub_w) {
+  for (int64_t k = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; k < n; k += int64_t(gridDim.x) * blockDim.x) {
+    const int32_t h = int32_t(row_key[k]);
+    const int32_t e = rowptr[hub_row[h]] + (vals[k] - hub_off[h]);
+    hub_col[k] = col[e];
+    if (hub_w) hub_w[k] = w[e];
+  }
+}
+
+// Chunk starts of one hub row, whose edges [a, b) of hub_col are sorted by source.  A band boundary (the source
+// crosses a multiple of 2^shift) is kept as a cut when the pieces on both sides hold at least `min_run` edges; every
+// piece between kept cuts is then cut into chunks of `thresh` edges.  emit(k, start) receives the k-th chunk start.
+template <typename F>
+__device__ int32_t hub_band_walk(const int32_t* __restrict__ hub_col, int32_t a, int32_t b, int shift, int32_t thresh,
+                                 int32_t min_run, F emit) {
+  int32_t k = 0, last = a, s = a;
+  while (s < b) {
+    const int64_t next = (int64_t(hub_col[s] >> shift) + 1) << shift;   // first source of the next band
+    int32_t lo = s, hi = b;                                              // first p in (s, b] with hub_col[p] >= next
+    while (lo < hi) {
+      const int32_t mid = lo + ((hi - lo) >> 1);
+      if (int64_t(hub_col[mid]) >= next) hi = mid; else lo = mid + 1;
+    }
+    const int32_t p = lo;
+    if (p < b && (p - last < min_run || b - p < min_run)) { s = p; continue; }
+    for (int32_t q = last; q < p; q += thresh) emit(k++, q);
+    last = s = p;
+  }
+  return k;
+}
+
+__global__ void hub_band_count_kernel(const int32_t* __restrict__ hub_col, const int32_t* __restrict__ hub_off,
+                                      int64_t n_hub, int shift, int32_t thresh, int32_t min_run,
+                                      int32_t* __restrict__ nch /* [n_hub+1] */) {
+  const int64_t h = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
+  if (h < n_hub) nch[h] = hub_band_walk(hub_col, hub_off[h], hub_off[h + 1], shift, thresh, min_run, [](int32_t, int32_t) {});
+  else if (h == n_hub) nch[h] = 0;
+}
+
+__global__ void hub_band_fill_kernel(const int32_t* __restrict__ hub_col, const int32_t* __restrict__ hub_off,
+                                     const int32_t* __restrict__ band_chunk_ptr, int64_t n_hub, int shift,
+                                     int32_t thresh, int32_t min_run, int32_t* __restrict__ cut, uint32_t* __restrict__ keys,
+                                     int32_t* __restrict__ vals) {
+  const int64_t h = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
+  if (h == n_hub) cut[band_chunk_ptr[n_hub]] = hub_off[n_hub];        // the end of the last chunk
+  if (h >= n_hub) return;
+  const int32_t c0 = band_chunk_ptr[h];
+  hub_band_walk(hub_col, hub_off[h], hub_off[h + 1], shift, thresh, min_run, [&](int32_t k, int32_t q) {
+    cut[c0 + k] = q;
+    keys[c0 + k] = uint32_t(hub_col[q] >> shift);                     // band of the chunk's first edge
+    vals[c0 + k] = c0 + k;
+  });
+}
+
 int bits_for(uint64_t n_keys) {  // number of key bits needed to represent values < n_keys
   int b = 1;
   while ((uint64_t(1) << b) < n_keys && b < 32) ++b;
@@ -561,6 +648,83 @@ int gmlm_hub_fill(const int32_t* rowptr, int64_t num_rows, int32_t thresh, int64
   hub_fill_chunks_kernel<<<int((threads + kThreads - 1) / kThreads), kThreads, 0, st>>>(
       rowptr, hub_row, hub_chunk_ptr, n_hub, thresh, chunk_beg, chunk_end);
   GMLM_LAUNCH_CHECK();
+  return GMLM_OK;
+}
+
+size_t gmlm_hub_band_workspace_bytes(int64_t n_hub_edges) {
+  if (n_hub_edges < 1) n_hub_edges = 1;
+  const size_t prim_bytes = std::max(sort_temp_bytes(n_hub_edges), scan_temp_bytes(n_hub_edges + 1));
+  return prim_bytes + 4 * (size_t(n_hub_edges) * 4 + 256) + 4096;
+}
+
+int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w, int64_t n_hub, const int32_t* hub_row,
+                       const int32_t* hub_off, int64_t n_hub_edges, int band_shift, int32_t thresh, int32_t min_run,
+                       int32_t* hub_col, float* hub_w, int32_t* band_chunk_ptr, int64_t* n_band_host, void* ws,
+                       size_t ws_bytes, void* stream) {
+  GMLM_REQUIRE(n_hub >= 0 && n_hub_edges >= 0 && n_hub_edges < (int64_t(1) << 31) - 1, "hub_band_sort: bad sizes");
+  GMLM_REQUIRE(band_shift >= 1 && band_shift <= 30 && thresh >= 1 && min_run >= 1, "hub_band_sort: bad band parameters");
+  GMLM_REQUIRE(ws_bytes >= gmlm_hub_band_workspace_bytes(n_hub_edges), "hub_band_sort: workspace too small");
+  *n_band_host = 0;
+  if (n_hub == 0) return GMLM_OK;
+  GMLM_REQUIRE(rowptr && col && hub_row && hub_off && hub_col && band_chunk_ptr && (hub_w == nullptr || w != nullptr),
+               "hub_band_sort: null pointer");
+  cudaStream_t st = as_stream(stream);
+  Carver cv(ws);
+  uint32_t* keys_a = cv.take<uint32_t>(n_hub_edges);
+  uint32_t* keys_b = cv.take<uint32_t>(n_hub_edges);
+  int32_t* vals_a = cv.take<int32_t>(n_hub_edges);
+  int32_t* vals_b = cv.take<int32_t>(n_hub_edges);
+  void* prim_ws = cv.take<char>(0);
+  const size_t prim_bytes = ws_bytes - cv.used();
+  // stable by source, then stable by hub row: each row's edges in source order, ties in CSR order
+  hub_band_keys_kernel<<<int((n_hub * 32 + kThreads - 1) / kThreads), kThreads, 0, st>>>(rowptr, col, hub_row, hub_off,
+                                                                                       n_hub, keys_a, vals_a);
+  GMLM_LAUNCH_CHECK();
+  if (int rc = prim::radix_sort_pairs(keys_a, vals_a, keys_b, vals_b, n_hub_edges, 31, prim_ws, prim_bytes, st)) return rc;
+  hub_band_rowkey_kernel<<<grid_for(n_hub_edges, 2), kThreads, 0, st>>>(vals_b, n_hub_edges, hub_off, n_hub, keys_b);
+  GMLM_LAUNCH_CHECK();
+  if (int rc = prim::radix_sort_pairs(keys_b, vals_b, keys_a, vals_a, n_hub_edges, bits_for(uint64_t(n_hub)), prim_ws,
+                                      prim_bytes, st))
+    return rc;
+  hub_band_gather_kernel<<<grid_for(n_hub_edges, 2), kThreads, 0, st>>>(keys_a, vals_a, n_hub_edges, rowptr, hub_row,
+                                                                        hub_off, col, w, hub_col, hub_w);
+  GMLM_LAUNCH_CHECK();
+  hub_band_count_kernel<<<int((n_hub + 1 + kThreads - 1) / kThreads), kThreads, 0, st>>>(
+      hub_col, hub_off, n_hub, band_shift, thresh, min_run, band_chunk_ptr);
+  GMLM_LAUNCH_CHECK();
+  if (int rc = prim::exclusive_scan_i32(band_chunk_ptr, band_chunk_ptr, n_hub + 1, prim_ws, prim_bytes, st)) return rc;
+  int32_t n_band = 0;
+  GMLM_CUDA_TRY(cudaMemcpyAsync(&n_band, band_chunk_ptr + n_hub, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  GMLM_CUDA_TRY(cudaStreamSynchronize(st));
+  *n_band_host = n_band;
+  return GMLM_OK;
+}
+
+int gmlm_hub_band_order(const int32_t* hub_col, const int32_t* hub_off, int64_t n_hub, int64_t n_hub_edges,
+                        int64_t n_band, int band_shift, int32_t thresh, int32_t min_run, int32_t* band_plan, void* ws,
+                        size_t ws_bytes, void* stream) {
+  GMLM_REQUIRE(n_hub >= 0 && n_band >= n_hub && n_band <= n_hub_edges, "hub_band_order: bad sizes");
+  GMLM_REQUIRE(band_shift >= 1 && band_shift <= 30 && thresh >= 1 && min_run >= 1, "hub_band_order: bad band parameters");
+  GMLM_REQUIRE(ws_bytes >= gmlm_hub_band_workspace_bytes(n_hub_edges), "hub_band_order: workspace too small");
+  if (n_hub == 0) return GMLM_OK;
+  GMLM_REQUIRE(hub_col && hub_off && band_plan, "hub_band_order: null pointer");
+  cudaStream_t st = as_stream(stream);
+  const int32_t* band_chunk_ptr = band_plan;
+  int32_t* cut = band_plan + n_hub + 1;
+  int32_t* order = cut + n_band + 1;
+  Carver cv(ws);
+  uint32_t* keys_a = cv.take<uint32_t>(n_band);
+  uint32_t* keys_b = cv.take<uint32_t>(n_band);
+  int32_t* vals_a = cv.take<int32_t>(n_band);
+  void* prim_ws = cv.take<char>(0);
+  const size_t prim_bytes = ws_bytes - cv.used();
+  hub_band_fill_kernel<<<int((n_hub + 1 + kThreads - 1) / kThreads), kThreads, 0, st>>>(
+      hub_col, hub_off, band_chunk_ptr, n_hub, band_shift, thresh, min_run, cut, keys_a, vals_a);
+  GMLM_LAUNCH_CHECK();
+  // stable by band: chunks of one band keep their row order
+  if (int rc = prim::radix_sort_pairs(keys_a, vals_a, keys_b, order, n_band, bits_for((uint64_t(0x7fffffff) >> band_shift) + 1),
+                                      prim_ws, prim_bytes, st))
+    return rc;
   return GMLM_OK;
 }
 

@@ -23,8 +23,12 @@
 //     Empty rows are written as zeros without touching the accumulator.
 //   * chunk kernel (hub path): rows longer than `hub_thresh` are cut into fixed chunks of
 //     hub_thresh edges, one group per chunk, fp32 partials, then an in-order final sum.
-//   * Determinism: fp32 accumulation strictly in CSR order (stable-sorted = original edge
-//     order), fixed chunking, no atomics: bit-identical run to run.
+//     Contiguous 512-byte rows (F = 256 bf16 / 128 fp32) run the band-ordered hub plan instead
+//     (gmlm_hub_band_sort): each hub row's edges sorted by source, chunks also cut where the
+//     source crosses a band of 2^17 rows, and the chunks launched band by band (chunk_order),
+//     so the rows of one band are gathered from L2 while that band's chunks run.
+//   * Determinism: fp32 accumulation in a fixed order (CSR order = original edge order; hub rows
+//     of the band plan in source order), fixed chunking, no atomics: bit-identical run to run.
 #include <cuda.h>
 
 #include <algorithm>
@@ -66,6 +70,7 @@ struct ChunkParams {
   int64_t feat;
   const int32_t* chunk_beg;
   const int32_t* chunk_end;
+  const int32_t* order;    // [n_chunks] chunk run by group i (nullptr = chunk i); the partial still goes to slot c
   const int32_t* col;
   const float* w;
   int64_t w_stride;
@@ -412,8 +417,9 @@ __global__ void __launch_bounds__(256, MINB) chunk_kernel(const ChunkParams p) {
   const int gl = lane % LPR;
   const int g = lane / LPR;
   const unsigned gmask = (LPR == 32) ? 0xffffffffu : (((1u << LPR) - 1u) << (g * LPR));
-  const int64_t c_id = (int64_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * GROUPS + g;
-  if (c_id >= p.n_chunks) return;
+  const int64_t g_id = (int64_t(blockIdx.x) * (blockDim.x >> 5) + (threadIdx.x >> 5)) * GROUPS + g;
+  if (g_id >= p.n_chunks) return;
+  const int64_t c_id = p.order ? __ldg(p.order + g_id) : g_id;
   const int64_t slab_stride = p.slab_stride ? p.slab_stride : int64_t(LPR) * VEC * CH;
   const int64_t slab_width = p.slab_width ? p.slab_width : slab_stride;
   const int64_t f0 = int64_t(blockIdx.y) * slab_stride + gl * VEC;
@@ -913,12 +919,13 @@ extern "C" int gmlm_group_plan(const int32_t* rowptr, int64_t num_rows, int64_t 
   return GMLM_OK;
 }
 
-extern "C" int gmlm_spmm_csr(const void* x, int dtype, int64_t feat, int64_t ldx, const int32_t* rowptr,
-                             const int32_t* col, const float* w, int32_t w_heads, int64_t num_rows, int mode,
-                             const int32_t* grp_row, int64_t n_groups, int32_t hub_thresh, int64_t n_hub,
-                             int64_t n_chunks, const int32_t* hub_row, const int32_t* hub_chunk_ptr,
-                             const int32_t* chunk_beg, const int32_t* chunk_end, float* hub_ws, void* out,
-                             int64_t ldo, void* stream) {
+extern "C" int gmlm_spmm_csr_banded(const void* x, int dtype, int64_t feat, int64_t ldx, const int32_t* rowptr,
+                                    const int32_t* col, const float* w, int32_t w_heads, int64_t num_rows, int mode,
+                                    const int32_t* grp_row, int64_t n_groups, int32_t hub_thresh, int64_t n_hub,
+                                    int64_t n_chunks, const int32_t* hub_row, const int32_t* hub_chunk_ptr,
+                                    const int32_t* chunk_beg, const int32_t* chunk_end, int64_t n_band,
+                                    const int32_t* band_plan, const int32_t* hub_col, const float* hub_w, float* hub_ws,
+                                    void* out, int64_t ldo, void* stream) {
   GMLM_REQUIRE(dtype == GMLM_F32 || dtype == GMLM_BF16, "spmm: dtype must be GMLM_F32 or GMLM_BF16");
   GMLM_REQUIRE(mode == GMLM_AGG_SUM || mode == GMLM_AGG_MEAN || mode == GMLM_AGG_WEIGHTED, "spmm: bad mode");
   GMLM_REQUIRE(feat >= 0 && num_rows >= 0 && ldx >= feat && ldo >= feat, "spmm: bad sizes");
@@ -932,6 +939,7 @@ extern "C" int gmlm_spmm_csr(const void* x, int dtype, int64_t feat, int64_t ldx
   GMLM_REQUIRE(x && rowptr && out, "spmm: null pointer");
   GMLM_REQUIRE(n_hub == 0 || (hub_row && hub_chunk_ptr && chunk_beg && chunk_end && hub_ws && hub_thresh >= 1),
                "spmm: hub plan arrays missing");
+  GMLM_REQUIRE(band_plan == nullptr || n_hub == 0 || (n_band >= n_hub && hub_col), "spmm: bad band plan");
   cudaStream_t st = as_stream(stream);
   const int esz = dtype == GMLM_F32 ? 4 : 2;
   const int fullvec = 16 / esz;
@@ -957,7 +965,20 @@ extern "C" int gmlm_spmm_csr(const void* x, int dtype, int64_t feat, int64_t ldx
   q.x = x; q.ldx = ldx; q.feat = feat;
   q.chunk_beg = chunk_beg; q.chunk_end = chunk_end; q.col = col; q.w = w;
   q.w_stride = w_heads; q.slab_stride = head_width; q.slab_width = head_width;
-  q.n_chunks = n_chunks; q.out = hub_ws;
+  q.n_chunks = n_chunks; q.out = hub_ws; q.order = nullptr;
+  // Contiguous rows of exactly 512 bytes, one weight column: the hub chunks of the band plan, run band by band, so
+  // that the rows one band of sources holds are gathered from L2 (DESIGN 4.1); a hub row is then summed in source
+  // order.  Every other width runs the CSR-order chunks of the hub plan.
+  const bool banded = band_plan && n_hub > 0 && (mode != GMLM_AGG_WEIGHTED || hub_w) && aligned &&
+                      feat * esz == 512 && ldx == feat && w_heads == 1;
+  if (banded) {
+    hub_chunk_ptr = band_plan;
+    q.chunk_beg = band_plan + n_hub + 1;
+    q.chunk_end = q.chunk_beg + 1;
+    q.order = q.chunk_beg + n_band + 1;
+    q.col = hub_col; q.w = hub_w;
+    q.n_chunks = n_band;
+  }
 
   // (Also measured and not kept: `prefetch.global.L2` of the rows the NEXT index batch gathers, issued by each lane while
   // the current batch is in flight -- bytes in flight towards L2 without registers: C5 forward 17.7 -> 18.8 ms in the
@@ -1005,4 +1026,15 @@ extern "C" int gmlm_spmm_csr(const void* x, int dtype, int64_t feat, int64_t ldx
     GMLM_CUDA_TRY(cudaStreamWaitEvent(st_rows, side->join, 0));
   }
   return GMLM_OK;
+}
+
+extern "C" int gmlm_spmm_csr(const void* x, int dtype, int64_t feat, int64_t ldx, const int32_t* rowptr,
+                             const int32_t* col, const float* w, int32_t w_heads, int64_t num_rows, int mode,
+                             const int32_t* grp_row, int64_t n_groups, int32_t hub_thresh, int64_t n_hub,
+                             int64_t n_chunks, const int32_t* hub_row, const int32_t* hub_chunk_ptr,
+                             const int32_t* chunk_beg, const int32_t* chunk_end, float* hub_ws, void* out,
+                             int64_t ldo, void* stream) {
+  return gmlm_spmm_csr_banded(x, dtype, feat, ldx, rowptr, col, w, w_heads, num_rows, mode, grp_row, n_groups,
+                              hub_thresh, n_hub, n_chunks, hub_row, hub_chunk_ptr, chunk_beg, chunk_end, 0, nullptr,
+                              nullptr, nullptr, hub_ws, out, ldo, stream);
 }

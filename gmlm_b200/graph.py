@@ -21,6 +21,12 @@ from . import _lib
 
 DEFAULT_HUB_THRESH = int(os.environ.get("GMLM_HUB_THRESH", "256"))
 DEFAULT_QUANTUM = int(os.environ.get("GMLM_GROUP_QUANTUM", "512"))   # 0 = uniform 32-row groups
+# Band-ordered hub plan (gmlm_hub_band_sort): a band is 2^HUB_BAND_SHIFT source rows, 64 MB of 512-byte rows, half
+# of the 126 MB L2.  Of 2^15 / 2^16 / 2^17 rows, 2^17 gave the fastest hub kernels on the C5 and C4 graphs
+# (DESIGN §4.1, profiles/r4_time_hub_chunks.jsonl).  A band boundary splits a chunk only when both pieces keep
+# HUB_BAND_MIN_RUN edges: shorter pieces cost a partial row written and read for few gathered rows.
+HUB_BAND_SHIFT = 17
+HUB_BAND_MIN_RUN = 32
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -52,6 +58,9 @@ class CSR:
     hub_chunk_ptr: Optional[torch.Tensor] = None
     chunk_beg: Optional[torch.Tensor] = None
     chunk_end: Optional[torch.Tensor] = None
+    hub_col: Optional[torch.Tensor] = None     # int32 [hub edges] col of the hub rows, each row sorted by source
+    hub_w: Optional[torch.Tensor] = None       # float32 [hub edges] w in the same order (weighted CSRs)
+    band_plan: Optional[torch.Tensor] = None   # int32 [band_chunk_ptr | cut | chunk_order] (include/gmlm_b200.h)
     quantum: int = 0                           # cost-balanced group plan (0 = uniform groups)
     n_groups: int = 0
     grp_row: Optional[torch.Tensor] = None     # int32 [n_groups+1]
@@ -108,6 +117,47 @@ class CSR:
                                              _stream(dev)), "hub_fill")
             else:
                 self.hub_row = self.hub_chunk_ptr = self.chunk_beg = self.chunk_end = None
+        self.plan_bands()
+        return self
+
+    @property
+    def n_band_chunks(self) -> int:
+        if self.band_plan is None:
+            return 0
+        return (int(self.band_plan.numel()) - self.n_hub - 2) // 2
+
+    def plan_bands(self, band_shift: int = HUB_BAND_SHIFT):
+        """The band-ordered hub plan next to the hub plan: every hub row's edges sorted by source, cut into chunks
+        at most ``hub_thresh`` long and at band boundaries, chunks ordered by band (``gmlm_hub_band_*``)."""
+        self.hub_col = self.hub_w = self.band_plan = None
+        if not self.n_hub:
+            return self
+        lib = _lib.load()
+        dev = self.rowptr.device
+        with torch.cuda.device(dev):
+            hr = self.hub_row.long()
+            lens = self.rowptr[hr + 1] - self.rowptr[hr]
+            hub_off = torch.zeros(self.n_hub + 1, dtype=torch.int32, device=dev)
+            torch.cumsum(lens, 0, out=hub_off[1:])
+            n_edges = int(hub_off[-1].item())
+            hub_col = torch.empty(n_edges, dtype=torch.int32, device=dev)
+            hub_w = torch.empty(n_edges, dtype=torch.float32, device=dev) if self.w is not None and self.w.dim() == 1 else None
+            chunk_ptr = torch.empty(self.n_hub + 1, dtype=torch.int32, device=dev)
+            ws_bytes = lib.gmlm_hub_band_workspace_bytes(n_edges)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            n_band = C.c_int64(0)
+            _lib.check(lib.gmlm_hub_band_sort(_ptr(self.rowptr), _ptr(self.col), _ptr(self.w if hub_w is not None else None),
+                                              self.n_hub, _ptr(self.hub_row), _ptr(hub_off), n_edges, int(band_shift),
+                                              self.hub_thresh, HUB_BAND_MIN_RUN, _ptr(hub_col), _ptr(hub_w),
+                                              _ptr(chunk_ptr), C.byref(n_band), _ptr(ws), ws_bytes, _stream(dev)),
+                       "hub_band_sort")
+            nb = int(n_band.value)
+            band_plan = torch.empty(self.n_hub + 2 + 2 * nb, dtype=torch.int32, device=dev)
+            band_plan[:self.n_hub + 1].copy_(chunk_ptr)
+            _lib.check(lib.gmlm_hub_band_order(_ptr(hub_col), _ptr(hub_off), self.n_hub, n_edges, nb, int(band_shift),
+                                               self.hub_thresh, HUB_BAND_MIN_RUN, _ptr(band_plan), _ptr(ws), ws_bytes,
+                                               _stream(dev)), "hub_band_order")
+        self.hub_col, self.hub_w, self.band_plan = hub_col, hub_w, band_plan
         return self
 
 

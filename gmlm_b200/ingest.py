@@ -85,7 +85,8 @@ def build_dropped_graph(edge_index: torch.Tensor, keep_mask: torch.Tensor, num_n
     return RelGraph.build(ei, et, num_nodes, num_relations, keep_mask=keep)
 
 
-_CSR_FIELDS = ("rowptr", "col", "w", "perm", "hub_row", "hub_chunk_ptr", "chunk_beg", "chunk_end", "grp_row")
+_CSR_FIELDS = ("rowptr", "col", "w", "perm", "hub_row", "hub_chunk_ptr", "chunk_beg", "chunk_end", "grp_row", "hub_col",
+               "hub_w", "band_plan")
 
 
 def save_rel_graph(graph: RelGraph, path: str) -> None:
@@ -109,7 +110,7 @@ def load_rel_graph(path: str, device) -> RelGraph:
         raise _lib.GmlmError("load_rel_graph: the graph lives on a CUDA device (no CPU path)")
 
     def unpack(d):
-        kw = {k: (d[k].to(dev) if d[k] is not None else None) for k in _CSR_FIELDS}
+        kw = {k: (d[k].to(dev) if d.get(k) is not None else None) for k in _CSR_FIELDS}   # files without a band plan: none
         return CSR(num_rows=d["num_rows"], hub_thresh=d["hub_thresh"], n_hub=d["n_hub"], n_chunks=d["n_chunks"],
                    quantum=d["quantum"], n_groups=d["n_groups"], **kw)
     return RelGraph(num_nodes=blob["num_nodes"], num_edges=blob["num_edges"], num_relations=blob["num_relations"],

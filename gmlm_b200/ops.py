@@ -52,7 +52,8 @@ _LIB = torch.library.Library("gmlm", "DEF")
 _LIB.define("degree_i32(Tensor index, int num_nodes) -> Tensor")
 _LIB.define("edge_type_bucket(Tensor src, Tensor deg, int[] bounds) -> Tensor")
 _LIB.define("spmm_csr(Tensor x, Tensor rowptr, Tensor col, Tensor? w, int num_rows, int mode, Tensor? grp_row, "
-            "int hub_thresh, Tensor? hub_row, Tensor? hub_chunk_ptr, Tensor? chunk_beg, Tensor? chunk_end) -> Tensor")
+            "int hub_thresh, Tensor? hub_row, Tensor? hub_chunk_ptr, Tensor? chunk_beg, Tensor? chunk_end, "
+            "Tensor? hub_col=None, Tensor? hub_w=None, Tensor? band_plan=None) -> Tensor")
 _LIB.define("colstats(Tensor x) -> (Tensor, Tensor)")
 _LIB.define("graphnorm_fwd(Tensor x, Tensor weight, Tensor bias, Tensor mean_scale, float eps, bool fuse_gelu) "
             "-> (Tensor, Tensor, Tensor)")
@@ -64,9 +65,12 @@ _LIB.define("layernorm_bwd(Tensor x, Tensor gy, Tensor mean, Tensor rstd, Tensor
 _LIB.define("soft_mask_fwd(Tensor x, Tensor mask, Tensor token, float beta) -> Tensor")
 _LIB.define("soft_mask_bwd(Tensor gy, Tensor mask, float beta, bool need_gx) -> (Tensor, Tensor)")
 # differentiable ops (autograd registered below with torch.library.register_autograd)
-# a CSR travels as eight (optional) tensors: rowptr, col, w, grp_row, hub_row, hub_chunk_ptr, chunk_beg, chunk_end
+# a CSR travels as eleven (optional) tensors: rowptr, col, w, grp_row, hub_row, hub_chunk_ptr, chunk_beg, chunk_end,
+# hub_col, hub_w, band_plan
 _CSR_ARGS = ("Tensor {p}rowptr, Tensor {p}col, Tensor? {p}w, Tensor? {p}grp, Tensor? {p}hub_row, "
-             "Tensor? {p}hub_chunk_ptr, Tensor? {p}chunk_beg, Tensor? {p}chunk_end")
+             "Tensor? {p}hub_chunk_ptr, Tensor? {p}chunk_beg, Tensor? {p}chunk_end, Tensor? {p}hub_col, "
+             "Tensor? {p}hub_w, Tensor? {p}band_plan")
+_NC = 11
 _LIB.define("rgcn_aggregate(Tensor x, " + _CSR_ARGS.format(p="f_") + ", " + _CSR_ARGS.format(p="b_") +
             ", int[] meta) -> Tensor")
 _LIB.define("plan_aggregate(Tensor rows, " + _CSR_ARGS.format(p="f_") + ", " + _CSR_ARGS.format(p="b_") +
@@ -105,7 +109,7 @@ def _edge_type_bucket(src: torch.Tensor, deg: torch.Tensor, bounds: Sequence[int
 
 # ------------------------------------------------------------------------------ A5 / A14
 def _spmm_csr(x, rowptr, col, w, num_rows, mode, grp_row, hub_thresh, hub_row, hub_chunk_ptr, chunk_beg, chunk_end,
-              out=None):
+              hub_col=None, hub_w=None, band_plan=None, out=None):
     lib = _lib.load()
     x = _rowmajor(x)
     feat = int(x.size(1))
@@ -113,6 +117,7 @@ def _spmm_csr(x, rowptr, col, w, num_rows, mode, grp_row, hub_thresh, hub_row, h
     n_hub = int(hub_row.numel()) if hub_row is not None else 0
     n_chunks = int(chunk_beg.numel()) if chunk_beg is not None else 0
     n_groups = int(grp_row.numel()) - 1 if grp_row is not None else 0
+    n_band = (int(band_plan.numel()) - n_hub - 2) // 2 if (band_plan is not None and n_hub) else 0
     w_heads = int(w.size(1)) if (w is not None and w.dim() == 2) else 1
     if col.numel() == 0 and mode == _lib.AGG_WEIGHTED:
         mode, w, w_heads = _lib.AGG_SUM, None, 1          # no edges: every row is empty, the result is zeros
@@ -121,13 +126,13 @@ def _spmm_csr(x, rowptr, col, w, num_rows, mode, grp_row, hub_thresh, hub_row, h
             out = torch.empty((num_rows, feat), dtype=x.dtype, device=dev)
         elif out.shape != (num_rows, feat) or out.dtype != x.dtype or not out.is_contiguous():
             raise _lib.GmlmError("spmm: `out` must be a contiguous [num_rows, feat] tensor of x's dtype")
-        hub_ws = torch.empty(n_chunks * feat, dtype=torch.float32, device=dev) if n_hub else None
-        _lib.check(lib.gmlm_spmm_csr(_ptr(x), _dtype_code(x, "spmm_csr"), feat, _ld(x), _ptr(rowptr), _ptr(col),
-                                     _ptr(w), w_heads, num_rows, mode, _ptr(grp_row), n_groups, hub_thresh, n_hub,
-                                     n_chunks,
-                                     _ptr(hub_row),
-                                     _ptr(hub_chunk_ptr), _ptr(chunk_beg), _ptr(chunk_end), _ptr(hub_ws), _ptr(out),
-                                     feat, _stream(dev)), "spmm_csr")
+        hub_ws = torch.empty(max(n_chunks, n_band) * feat, dtype=torch.float32, device=dev) if n_hub else None
+        _lib.check(lib.gmlm_spmm_csr_banded(_ptr(x), _dtype_code(x, "spmm_csr"), feat, _ld(x), _ptr(rowptr), _ptr(col),
+                                            _ptr(w), w_heads, num_rows, mode, _ptr(grp_row), n_groups, hub_thresh, n_hub,
+                                            n_chunks, _ptr(hub_row), _ptr(hub_chunk_ptr), _ptr(chunk_beg),
+                                            _ptr(chunk_end), n_band, _ptr(band_plan if n_band else None),
+                                            _ptr(hub_col), _ptr(hub_w), _ptr(hub_ws), _ptr(out), feat, _stream(dev)),
+                   "spmm_csr")
     return out
 
 
@@ -135,13 +140,15 @@ def spmm(x: torch.Tensor, csr: CSR, mode: int, out: Optional[torch.Tensor] = Non
     """out[r] = reduce over row r of csr (no autograd).  ``out`` lets the result land in a caller-owned
     buffer (e.g. NVLink-peer-visible symmetric memory for the halo exchange)."""
     _require_cuda(x, "x")
+    weighted = mode == _lib.AGG_WEIGHTED
     if out is not None:
-        return _spmm_csr(x, csr.rowptr, csr.col, csr.w if mode == _lib.AGG_WEIGHTED else None, csr.num_rows, mode,
+        return _spmm_csr(x, csr.rowptr, csr.col, csr.w if weighted else None, csr.num_rows, mode,
                          csr.grp_row, csr.hub_thresh, csr.hub_row, csr.hub_chunk_ptr, csr.chunk_beg, csr.chunk_end,
-                         out=out)
-    return torch.ops.gmlm.spmm_csr(x, csr.rowptr, csr.col, csr.w if mode == _lib.AGG_WEIGHTED else None,
+                         csr.hub_col, csr.hub_w if weighted else None, csr.band_plan, out=out)
+    return torch.ops.gmlm.spmm_csr(x, csr.rowptr, csr.col, csr.w if weighted else None,
                                    csr.num_rows, mode, csr.grp_row, csr.hub_thresh, csr.hub_row, csr.hub_chunk_ptr,
-                                   csr.chunk_beg, csr.chunk_end)
+                                   csr.chunk_beg, csr.chunk_end, csr.hub_col, csr.hub_w if weighted else None,
+                                   csr.band_plan)
 
 
 # ------------------------------------------------------------------------------ A7
@@ -356,25 +363,27 @@ _LIB.impl("soft_mask_bwd", _soft_mask_bwd, "CUDA")
 # backward (torch.library.register_autograd) and a fake implementation (register_fake), so they can be called,
 # traced and differentiated as ordinary torch operators; the thin functions further down only validate arguments.
 def csr_pack(csr: CSR):
-    """CSR -> (Tensor?[8], [num_rows, hub_thresh]): rowptr, col, w, grp_row, hub_row, hub_chunk_ptr, chunk_beg, chunk_end."""
-    return ([csr.rowptr, csr.col, csr.w, csr.grp_row, csr.hub_row, csr.hub_chunk_ptr, csr.chunk_beg, csr.chunk_end],
-            [int(csr.num_rows), int(csr.hub_thresh)])
+    """CSR -> (Tensor?[11], [num_rows, hub_thresh]): rowptr, col, w, grp_row, hub_row, hub_chunk_ptr, chunk_beg,
+    chunk_end, hub_col, hub_w, band_plan."""
+    return ([csr.rowptr, csr.col, csr.w, csr.grp_row, csr.hub_row, csr.hub_chunk_ptr, csr.chunk_beg, csr.chunk_end,
+             csr.hub_col, csr.hub_w, csr.band_plan], [int(csr.num_rows), int(csr.hub_thresh)])
 
 
 def _spmm_list(x, c, rows, thresh, mode):
-    return _spmm_csr(x, c[0], c[1], c[2] if mode == _lib.AGG_WEIGHTED else None, rows, mode, c[3], thresh, c[4], c[5],
-                     c[6], c[7])
+    weighted = mode == _lib.AGG_WEIGHTED
+    return _spmm_csr(x, c[0], c[1], c[2] if weighted else None, rows, mode, c[3], thresh, c[4], c[5], c[6], c[7], c[8],
+                     c[9] if weighted else None, c[10])
 
 
 def _rgcn_aggregate_impl(x, *a):
-    fwd, meta = a[0:8], a[16]
+    fwd, meta = a[0:_NC], a[2 * _NC]
     rows_f, thresh_f, _, _, n_nodes, n_slots = meta
     h = _spmm_list(x, fwd, rows_f, thresh_f, _lib.AGG_MEAN)                 # [N*S, F]
     return h.view(n_nodes, n_slots * x.size(1))
 
 
 def _plan_aggregate_impl(rows, *a):
-    fwd, meta = a[0:8], a[16]
+    fwd, meta = a[0:_NC], a[2 * _NC]
     return _spmm_list(rows, fwd, meta[0], meta[1], _lib.AGG_WEIGHTED)
 
 
@@ -429,7 +438,8 @@ def _(src, deg, bounds):
 
 
 @torch.library.register_fake("gmlm::spmm_csr")
-def _(x, rowptr, col, w, num_rows, mode, grp_row, hub_thresh, hub_row, hub_chunk_ptr, chunk_beg, chunk_end):
+def _(x, rowptr, col, w, num_rows, mode, grp_row, hub_thresh, hub_row, hub_chunk_ptr, chunk_beg, chunk_end,
+      hub_col=None, hub_w=None, band_plan=None):
     return x.new_empty((num_rows, x.size(1)))
 
 
@@ -476,13 +486,13 @@ def _(gy, mask, beta, need_gx):
 
 @torch.library.register_fake("gmlm::rgcn_aggregate")
 def _(x, *a):
-    meta = a[16]
+    meta = a[2 * _NC]
     return x.new_empty((meta[4], meta[5] * x.size(1)))
 
 
 @torch.library.register_fake("gmlm::plan_aggregate")
 def _(rows, *a):
-    return rows.new_empty((a[16][0], rows.size(1)))
+    return rows.new_empty((a[2 * _NC][0], rows.size(1)))
 
 
 @torch.library.register_fake("gmlm::gemm_nt")
@@ -500,7 +510,7 @@ def _(row, col, rel, keep, num_rows, num_cols, num_relations, slot_of_rel, num_s
 # ---- autograd formulas
 def _rgcn_aggregate_setup(ctx, inputs, output):
     x = inputs[0]
-    ctx.bwd, ctx.meta, ctx.x_dtype = inputs[9:17], inputs[17], x.dtype
+    ctx.bwd, ctx.meta, ctx.x_dtype = inputs[1 + _NC:1 + 2 * _NC], inputs[1 + 2 * _NC], x.dtype
 
 
 def _rgcn_aggregate_backward(ctx, gh):
@@ -511,12 +521,12 @@ def _rgcn_aggregate_backward(ctx, gh):
     feat = gh.size(1) // n_slots
     b = ctx.bwd
     gx = torch.ops.gmlm.spmm_csr(gh.view(n_nodes * n_slots, feat), b[0], b[1], b[2], rows_b, _lib.AGG_WEIGHTED, b[3],
-                                 thresh_b, b[4], b[5], b[6], b[7])            # A14: gather on the transposed CSR
-    return (gx,) + (None,) * 17
+                                 thresh_b, b[4], b[5], b[6], b[7], b[8], b[9], b[10])   # A14: gather on the transposed CSR
+    return (gx,) + (None,) * (2 * _NC + 1)
 
 
 def _plan_aggregate_setup(ctx, inputs, output):
-    ctx.bwd, ctx.meta, ctx.in_dtype = inputs[9:17], inputs[17], inputs[0].dtype
+    ctx.bwd, ctx.meta, ctx.in_dtype = inputs[1 + _NC:1 + 2 * _NC], inputs[1 + 2 * _NC], inputs[0].dtype
 
 
 def _plan_aggregate_backward(ctx, g):
@@ -525,7 +535,7 @@ def _plan_aggregate_backward(ctx, g):
         g = g.to(ctx.in_dtype)
     b = ctx.bwd
     return (torch.ops.gmlm.spmm_csr(g, b[0], b[1], b[2], ctx.meta[2], _lib.AGG_WEIGHTED, b[3], ctx.meta[3], b[4], b[5],
-                                    b[6], b[7]),) + (None,) * 17
+                                    b[6], b[7], b[8], b[9], b[10]),) + (None,) * (2 * _NC + 1)
 
 
 def _graphnorm_setup(ctx, inputs, output):
@@ -954,7 +964,7 @@ class _RGCNSegCompact(torch.autograd.Function):
         S, fi, fo = len(live), weight.size(1), weight.size(2)
         h_c = _spmm_csr(x, plan.fwd.rowptr, plan.fwd.col, None, plan.fwd.num_rows, _lib.AGG_MEAN, plan.fwd.grp_row,
                         plan.fwd.hub_thresh, plan.fwd.hub_row, plan.fwd.hub_chunk_ptr, plan.fwd.chunk_beg,
-                        plan.fwd.chunk_end)
+                        plan.fwd.chunk_end, plan.fwd.hub_col, None, plan.fwd.band_plan)
         hq = _tma_rows(h_c, op_dtype)
         xq = _tma_rows(x[:num_nodes], op_dtype)
         wn, wt = basis_compose(weight, comp, root, live, op_dtype, "agg")
@@ -1006,7 +1016,8 @@ class _RGCNSegCompact(torch.autograd.Function):
                 dx = torch.zeros((ctx.num_src, fi), dtype=acc_dt, device=g.device)
             else:
                 dx = _spmm_csr(dh_c, b.rowptr, b.col, b.w, b.num_rows, _lib.AGG_WEIGHTED, b.grp_row, b.hub_thresh,
-                               b.hub_row, b.hub_chunk_ptr, b.chunk_beg, b.chunk_end)      # [num_src, Fi]
+                               b.hub_row, b.hub_chunk_ptr, b.chunk_beg, b.chunk_end, b.hub_col, b.hub_w,
+                               b.band_plan)                                              # [num_src, Fi]
             dxr = gemm_nt(gq, wn[S * fi:], out_dtype=acc_dt)                              # root term, local rows
             if dx.size(0) == dxr.size(0):
                 dx = dx + dxr

@@ -127,6 +127,26 @@ int gmlm_hub_fill(const int32_t* rowptr, int64_t num_rows, int32_t thresh, int64
                   int32_t* hub_row, int32_t* hub_chunk_ptr, int32_t* chunk_beg, int32_t* chunk_end,
                   void* ws, size_t ws_bytes, void* stream);
 
+/* ---- band-ordered hub plan (512-byte rows of gmlm_spmm_csr_banded) ----
+ * The edges of every hub row sorted by source (stable: ties keep CSR order), so that the chunks gathering from one
+ * band of 2^band_shift source rows can run together and find those rows in L2.
+ * hub_off[n_hub+1]: hub_off[h] = edges of hub rows before h (exclusive scan of the hub row lengths).
+ * band_sort : hub_col[n_hub_edges] (and hub_w, when w is given) = col / w of the hub rows, row by row, each row by
+ *             source; band_chunk_ptr[n_hub+1] = the row -> chunk pointer of the band cuts; *n_band_host = #chunks.
+ *             A band boundary inside a row is a cut when both sides hold >= min_run edges; pieces between cuts are
+ *             cut every `thresh` edges.
+ * band_order: band_plan = [band_chunk_ptr (n_hub+1, copied in by the caller) | cut (n_band+1) | chunk_order (n_band)];
+ *             chunk c covers hub_col[cut[c], cut[c+1]); chunk_order = chunk ids stably sorted by the band of their
+ *             first edge. */
+size_t gmlm_hub_band_workspace_bytes(int64_t n_hub_edges);
+int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w, int64_t n_hub, const int32_t* hub_row,
+                       const int32_t* hub_off, int64_t n_hub_edges, int band_shift, int32_t thresh, int32_t min_run,
+                       int32_t* hub_col, float* hub_w, int32_t* band_chunk_ptr, int64_t* n_band_host, void* ws,
+                       size_t ws_bytes, void* stream);
+int gmlm_hub_band_order(const int32_t* hub_col, const int32_t* hub_off, int64_t n_hub, int64_t n_hub_edges,
+                        int64_t n_band, int band_shift, int32_t thresh, int32_t min_run, int32_t* band_plan, void* ws,
+                        size_t ws_bytes, void* stream);
+
 /* ---- cost-balanced group plan for gmlm_spmm_csr ----
  * Cuts the row sequence where (r + rowptr[r]) crosses multiples of `quantum`, so that every
  * group of lanes moves about `quantum` row-sized units (one per gathered edge + one per written
@@ -149,6 +169,18 @@ int gmlm_spmm_csr(const void* x, int dtype, int64_t feat, int64_t ldx,
                   int32_t hub_thresh, int64_t n_hub, int64_t n_chunks, const int32_t* hub_row,
                   const int32_t* hub_chunk_ptr, const int32_t* chunk_beg, const int32_t* chunk_end,
                   float* hub_ws, void* out, int64_t ldo, void* stream);
+/* gmlm_spmm_csr with the band-ordered hub plan (gmlm_hub_band_sort / _order) of the same CSR: rows of exactly 512
+ * bytes (F = 256 bf16 / 128 fp32, no head slabs, one weight column) gather their hub chunks from hub_col / hub_w in
+ * chunk_order, so that one band of source rows is served from L2; other widths use the chunk plan above.  band_plan
+ * NULL (or hub_w NULL in weighted mode) = the chunk plan above for every width.  hub_ws holds
+ * max(n_chunks, n_band) * feat floats.  gmlm_spmm_csr is this call without a band plan. */
+int gmlm_spmm_csr_banded(const void* x, int dtype, int64_t feat, int64_t ldx,
+                         const int32_t* rowptr, const int32_t* col, const float* w, int32_t w_heads,
+                         int64_t num_rows, int mode, const int32_t* grp_row, int64_t n_groups,
+                         int32_t hub_thresh, int64_t n_hub, int64_t n_chunks, const int32_t* hub_row,
+                         const int32_t* hub_chunk_ptr, const int32_t* chunk_beg, const int32_t* chunk_end,
+                         int64_t n_band, const int32_t* band_plan, const int32_t* hub_col, const float* hub_w,
+                         float* hub_ws, void* out, int64_t ldo, void* stream);
 
 /* ---- A7  GraphNorm  [PyG] torch_geometric.nn.GraphNorm(batch=None), called main.py:273,286,299,309 ----
  * stats: colsum[c] = sum_i x[i,c], colsq[c] = sum_i x[i,c]^2 in fp64 (deterministic two-stage).
