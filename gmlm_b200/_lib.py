@@ -76,7 +76,13 @@ SIGNATURES = {
                                   _p, _p, _p, _p, _p, _sz, _p, _i64, _p, _p, _p]),
     "gmlm_gat_bwd_edges": (_int, [_p, _p, _i64, _p, _int, _i64, _p, _i64, _p, _p, _p, _p, _p, _int, _int, _f32, _f32,
                                   C.c_uint64, _i32, _i64, _i64, _p, _p, _p, _p, _p, _sz, _p, _p, _p, _p]),
+    "gmlm_gat_fused_fwd_eattr": (_int, [_p, _p, _i64, _p, _int, _i64, _p, _p, _p, _int, _int, _f32, _f32, C.c_uint64, _i32,
+                                        _i64, _i64, _p, _p, _p, _p, _p, _sz, _p, _i64, _p, _p, _p]),
+    "gmlm_gat_bwd_edges_eattr": (_int, [_p, _p, _i64, _p, _int, _i64, _p, _i64, _p, _p, _p, _p, _p, _p, _int, _int, _f32,
+                                        _f32, C.c_uint64, _i32, _i64, _i64, _p, _p, _p, _p, _p, _sz, _p, _p, _p, _p]),
     "gmlm_gat_dropout_mask": (_int, [C.c_uint64, _i64, _f32, _p, _p]),
+    "gmlm_gat_loop_fill": (_int, [_p, _p, _p, _p, _i64, _int, _p, _p]),
+    "gmlm_gat_loop_fill_bwd": (_int, [_p, _p, _p, _p, _p, _i64, _int, _p, _p]),
     "gmlm_segment_sum_f32": (_int, [_p, _p, _p, _i64, _int, _p, _p]),
     "gmlm_gather_rows": (_int, [_p, _int, _i64, _i64, _p, _i64, _p, _i64, _p]),
     "gmlm_scatter_add_rows": (_int, [_p, _int, _i64, _i64, _p, _i64, _p, _i64, _p]),

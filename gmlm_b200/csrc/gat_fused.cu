@@ -4,6 +4,12 @@
 //   out[i,h,:] = sum_{e -> i} alpha[e,h] * z[src_e,h,:],
 //   alpha[e,h] = exp(s[e,h] - max_i) / (sum_i exp(s - max_i) + 1e-16),   s[e,h] = leaky_relu(a_src[src_e,h] + a_dst[i,h])
 //
+// Edge features (upstream GATConv(edge_dim)): the `_eattr` entry points take a_edge [nnz, H], a per-(edge, head)
+// score term in CSR order (loop entries included), read where a_src is read and added before the leaky ReLU:
+// s[e,h] = leaky_relu((a_src[src_e,h] + a_edge[e,h]) + a_dst[i,h]), in the forward scan and in the backward's
+// recomputed score alike.  Its gradient is d_score, which the backward edge pass writes anyway.  The term is the
+// template flag E, so the instantiations without it (a_edge = NULL) carry no code for it.
+//
 // Forward = ONE pass over the in-edges of a destination row with an ONLINE softmax: the score is computed where
 // the source row is gathered, the running maximum m, normaliser l and the fp32 accumulator are rescaled by
 // exp(m_old - m_new) whenever the maximum grows, and alpha is never written (round 1: three passes over the scores
@@ -63,6 +69,7 @@ struct GatParams {
   float slope, p_drop;
   uint64_t seed;
   int32_t hub_thresh;
+  const float* a_edge;  // [nnz, H] in CSR order, read only by the E = true instantiations
 };
 
 template <typename T, int VEC, int CH, bool G>
@@ -88,7 +95,7 @@ struct Lane {
 };
 
 // online-softmax scan of edges [b, e) of destination row `row`
-template <typename T, int VEC, int CH, bool G>
+template <typename T, int VEC, int CH, bool G, bool E>
 __device__ __forceinline__ void gat_scan(const GatParams& p, const Lane<T, VEC, CH, G>& ln, int64_t row, int32_t b, int32_t e,
                                          float (&m)[CH], float (&l)[CH], float (&acc)[CH][VEC]) {
   const T* __restrict__ z = static_cast<const T*>(p.z);
@@ -110,9 +117,11 @@ __device__ __forceinline__ void gat_scan(const GatParams& p, const Lane<T, VEC, 
     for (int ch = 0; ch < CH; ++ch) {
       if (!ln.valid[ch]) continue;
       as0[ch] = __ldg(p.a_src + int64_t(s0) * p.H + ln.head[ch]);
+      if constexpr (E) as0[ch] += __ldg(p.a_edge + int64_t(k) * p.H + ln.head[ch]);
       z0[ch].load(z + int64_t(s0) * p.ldz + ln.f[ch]);
       if (two) {
         as1[ch] = __ldg(p.a_src + int64_t(s1) * p.H + ln.head[ch]);
+        if constexpr (E) as1[ch] += __ldg(p.a_edge + int64_t(k + 1) * p.H + ln.head[ch]);
         z1[ch].load(z + int64_t(s1) * p.ldz + ln.f[ch]);
       }
     }
@@ -139,7 +148,7 @@ __device__ __forceinline__ void gat_scan(const GatParams& p, const Lane<T, VEC, 
   }
 }
 
-template <typename T, int VEC, int CH, bool G>
+template <typename T, int VEC, int CH, bool G, bool E>
 __global__ void __launch_bounds__(256) gat_rows_kernel(const GatParams p, int64_t num_rows, T* __restrict__ out,
                                                        int64_t ldo, float* __restrict__ m_out, float* __restrict__ l_out) {
   const int64_t r = (int64_t(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
@@ -150,7 +159,7 @@ __global__ void __launch_bounds__(256) gat_rows_kernel(const GatParams p, int64_
   Lane<T, VEC, CH, G> ln;
   ln.init(lane, p);
   float m[CH], l[CH], acc[CH][VEC];
-  gat_scan<T, VEC, CH, G>(p, ln, r, b, e, m, l, acc);
+  gat_scan<T, VEC, CH, G, E>(p, ln, r, b, e, m, l, acc);
   const float keep_scale = p.p_drop > 0.f ? 1.0f / (1.0f - p.p_drop) : 1.0f;
 #pragma unroll
   for (int ch = 0; ch < CH; ++ch) {
@@ -169,7 +178,7 @@ __global__ void __launch_bounds__(256) gat_rows_kernel(const GatParams p, int64_
   }
 }
 
-template <typename T, int VEC, int CH, bool G>
+template <typename T, int VEC, int CH, bool G, bool E>
 __global__ void __launch_bounds__(256) gat_chunk_kernel(const GatParams p, const int32_t* __restrict__ chunk_beg,
                                                         const int32_t* __restrict__ chunk_end,
                                                         const int32_t* __restrict__ chunk_row, int64_t n_chunks,
@@ -181,7 +190,7 @@ __global__ void __launch_bounds__(256) gat_chunk_kernel(const GatParams p, const
   Lane<T, VEC, CH, G> ln;
   ln.init(lane, p);
   float m[CH], l[CH], acc[CH][VEC];
-  gat_scan<T, VEC, CH, G>(p, ln, __ldg(chunk_row + c), __ldg(chunk_beg + c), __ldg(chunk_end + c), m, l, acc);
+  gat_scan<T, VEC, CH, G, E>(p, ln, __ldg(chunk_row + c), __ldg(chunk_beg + c), __ldg(chunk_end + c), m, l, acc);
   const int64_t hc = int64_t(p.H) * p.C;
 #pragma unroll
   for (int ch = 0; ch < CH; ++ch) {
@@ -232,7 +241,7 @@ __global__ void chunk_rows_kernel(const int32_t* __restrict__ hub_row, const int
 
 // ---------------------------------------------------------------------------------- backward, edge pass
 // one warp per (row | chunk): alpha_eff[k,h], d_score[k,h] for its edges, partial da_dst[., h]
-template <typename T, int VEC, int CH, bool G>
+template <typename T, int VEC, int CH, bool G, bool E>
 __device__ __forceinline__ void gat_bwd_scan(const GatParams& p, const Lane<T, VEC, CH, G>& ln, int lane, int64_t row,
                                              int32_t b, int32_t e, const T* __restrict__ g, int64_t ldg,
                                              const float* __restrict__ m_in, const float* __restrict__ l_in,
@@ -283,7 +292,9 @@ __device__ __forceinline__ void gat_bwd_scan(const GatParams& p, const Lane<T, V
     }
     if (lane < nh) {
       const int hd = G ? hh : lane;                    // this lane's head (global index)
-      const float raw = __ldg(p.a_src + int64_t(s) * p.H + hd) + ad;
+      float as = __ldg(p.a_src + int64_t(s) * p.H + hd);
+      if constexpr (E) as += __ldg(p.a_edge + int64_t(k) * p.H + hd);   // summed as in the forward's scan
+      const float raw = as + ad;
       const float alpha = expf(lrelu(raw, p.slope) - mm) * inv_l;
       const bool keep = p.p_drop <= 0.f || drop_keep(p.seed, uint64_t(k) * p.H + hd, p.p_drop);
       const float ks = keep ? keep_scale : 0.f;
@@ -297,7 +308,7 @@ __device__ __forceinline__ void gat_bwd_scan(const GatParams& p, const Lane<T, V
   if (lane < nh) da_dst_out[G ? hh : lane] = dsum;
 }
 
-template <typename T, int VEC, int CH, bool G>
+template <typename T, int VEC, int CH, bool G, bool E>
 __global__ void __launch_bounds__(256) gat_bwd_rows_kernel(const GatParams p, int64_t num_rows, const T* __restrict__ g,
                                                            int64_t ldg, const float* __restrict__ m_in,
                                                            const float* __restrict__ l_in, const float* __restrict__ t_in,
@@ -310,10 +321,10 @@ __global__ void __launch_bounds__(256) gat_bwd_rows_kernel(const GatParams p, in
   if (e - b > p.hub_thresh) return;
   Lane<T, VEC, CH, G> ln;
   ln.init(lane, p);
-  gat_bwd_scan<T, VEC, CH, G>(p, ln, lane, r, b, e, g, ldg, m_in, l_in, t_in, alpha_eff, d_score, da_dst + r * p.H);
+  gat_bwd_scan<T, VEC, CH, G, E>(p, ln, lane, r, b, e, g, ldg, m_in, l_in, t_in, alpha_eff, d_score, da_dst + r * p.H);
 }
 
-template <typename T, int VEC, int CH, bool G>
+template <typename T, int VEC, int CH, bool G, bool E>
 __global__ void __launch_bounds__(256) gat_bwd_chunk_kernel(const GatParams p, const int32_t* __restrict__ chunk_beg,
                                                             const int32_t* __restrict__ chunk_end,
                                                             const int32_t* __restrict__ chunk_row, int64_t n_chunks,
@@ -326,7 +337,7 @@ __global__ void __launch_bounds__(256) gat_bwd_chunk_kernel(const GatParams p, c
   if (c >= n_chunks) return;
   Lane<T, VEC, CH, G> ln;
   ln.init(lane, p);
-  gat_bwd_scan<T, VEC, CH, G>(p, ln, lane, __ldg(chunk_row + c), __ldg(chunk_beg + c), __ldg(chunk_end + c), g, ldg, m_in,
+  gat_bwd_scan<T, VEC, CH, G, E>(p, ln, lane, __ldg(chunk_row + c), __ldg(chunk_beg + c), __ldg(chunk_end + c), g, ldg, m_in,
                            l_in, t_in, alpha_eff, d_score, da_part + c * p.H);
 }
 
@@ -378,15 +389,24 @@ int dispatch_geo(int dtype, int64_t hc, bool aligned, Fn&& fn) {
 }
 
 // a row that fits one warp: the instantiation for its width, no group offsets (G = false); a row cut into head groups:
-// the widest instantiation of its path (G = true)
-template <typename Fn>
-int dispatch_gat(int dtype, int64_t hc, bool aligned, int n_groups, Fn&& fn) {
+// the widest instantiation of its path (G = true).  E: the per-edge score term a_edge is read (a compile-time flag,
+// so the instantiations without it are the code that runs when no term is passed)
+template <bool E, typename Fn>
+int dispatch_gat_e(int dtype, int64_t hc, bool aligned, int n_groups, Fn&& fn) {
   if (n_groups == 1)
     return dispatch_geo(dtype, hc, aligned, [&]<typename T, int VEC, int CH>() -> int {
-      return fn.template operator()<T, VEC, CH, false>();
+      return fn.template operator()<T, VEC, CH, false, E>();
     });
-  if (dtype == GMLM_F32) return aligned ? fn.template operator()<float, 4, 8, true>() : fn.template operator()<float, 1, 8, true>();
-  return aligned ? fn.template operator()<__nv_bfloat16, 8, 4, true>() : fn.template operator()<__nv_bfloat16, 1, 8, true>();
+  if (dtype == GMLM_F32)
+    return aligned ? fn.template operator()<float, 4, 8, true, E>() : fn.template operator()<float, 1, 8, true, E>();
+  return aligned ? fn.template operator()<__nv_bfloat16, 8, 4, true, E>()
+                 : fn.template operator()<__nv_bfloat16, 1, 8, true, E>();
+}
+
+template <typename Fn>
+int dispatch_gat(int dtype, int64_t hc, bool aligned, int n_groups, bool edge, Fn&& fn) {
+  return edge ? dispatch_gat_e<true>(dtype, hc, aligned, n_groups, fn)
+              : dispatch_gat_e<false>(dtype, hc, aligned, n_groups, fn);
 }
 
 inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
@@ -420,12 +440,13 @@ extern "C" size_t gmlm_gat_workspace_bytes(int64_t n_chunks, int heads, int head
   return size_t(n_chunks) * (4 + size_t(heads) * 8 + size_t(heads) * head_dim * 4) + 1024;
 }
 
-extern "C" int gmlm_gat_fused_fwd(const int32_t* rowptr, const int32_t* col, int64_t num_rows, const void* z, int dtype,
-                                  int64_t ldz, const float* a_src, const float* a_dst, int heads, int head_dim,
-                                  float negative_slope, float p_drop, uint64_t seed, int32_t hub_thresh, int64_t n_hub,
-                                  int64_t n_chunks, const int32_t* hub_row, const int32_t* hub_chunk_ptr,
-                                  const int32_t* chunk_beg, const int32_t* chunk_end, void* ws, size_t ws_bytes,
-                                  void* out, int64_t ldo, float* m_out, float* l_out, void* stream) {
+extern "C" int gmlm_gat_fused_fwd_eattr(const int32_t* rowptr, const int32_t* col, int64_t num_rows, const void* z,
+                                        int dtype, int64_t ldz, const float* a_src, const float* a_dst,
+                                        const float* a_edge, int heads, int head_dim, float negative_slope,
+                                        float p_drop, uint64_t seed, int32_t hub_thresh, int64_t n_hub,
+                                        int64_t n_chunks, const int32_t* hub_row, const int32_t* hub_chunk_ptr,
+                                        const int32_t* chunk_beg, const int32_t* chunk_end, void* ws, size_t ws_bytes,
+                                        void* out, int64_t ldo, float* m_out, float* l_out, void* stream) {
   GMLM_REQUIRE(dtype == GMLM_F32 || dtype == GMLM_BF16, "gat_fused_fwd: dtype must be GMLM_F32 or GMLM_BF16");
   GMLM_REQUIRE(num_rows >= 0 && heads >= 1 && heads <= 32 && head_dim >= 1, "gat_fused_fwd: bad sizes (1..32 heads)");
   GMLM_REQUIRE(p_drop >= 0.f && p_drop < 1.f, "gat_fused_fwd: dropout must be in [0, 1)");
@@ -442,7 +463,7 @@ extern "C" int gmlm_gat_fused_fwd(const int32_t* rowptr, const int32_t* col, int
   if (int rc = head_groups(heads, head_dim, aligned, "gat_fused_fwd", &hgp)) return rc;
   cudaStream_t st = as_stream(stream);
   GatParams p{rowptr, col, z, ldz, a_src, a_dst, heads, head_dim, hgp.hg, negative_slope, p_drop, seed,
-              n_hub > 0 ? hub_thresh : 0x7fffffff};
+              n_hub > 0 ? hub_thresh : 0x7fffffff, a_edge};
   Carver cv(ws);
   int32_t* chunk_row = n_hub ? cv.take<int32_t>(n_chunks) : nullptr;
   float* pm = n_hub ? cv.take<float>(n_chunks * heads) : nullptr;
@@ -450,13 +471,14 @@ extern "C" int gmlm_gat_fused_fwd(const int32_t* rowptr, const int32_t* col, int
   float* pacc = n_hub ? cv.take<float>(n_chunks * hc) : nullptr;
   const dim3 grid(unsigned((num_rows * 32 + 255) / 256), unsigned(hgp.n));
   const dim3 cgrid(unsigned((n_chunks * 32 + 255) / 256), unsigned(hgp.n));
-  int rc = dispatch_gat(dtype, hc, aligned, hgp.n, [&]<typename T, int VEC, int CH, bool G>() -> int {
-    gat_rows_kernel<T, VEC, CH, G><<<grid, 256, 0, st>>>(p, num_rows, static_cast<T*>(out), ldo, m_out, l_out);
+  const bool edge = a_edge != nullptr;
+  int rc = dispatch_gat(dtype, hc, aligned, hgp.n, edge, [&]<typename T, int VEC, int CH, bool G, bool E>() -> int {
+    gat_rows_kernel<T, VEC, CH, G, E><<<grid, 256, 0, st>>>(p, num_rows, static_cast<T*>(out), ldo, m_out, l_out);
     GMLM_LAUNCH_CHECK();
     if (n_hub) {
       chunk_rows_kernel<<<unsigned(n_hub), 128, 0, st>>>(hub_row, hub_chunk_ptr, n_hub, chunk_row);
       GMLM_LAUNCH_CHECK();
-      gat_chunk_kernel<T, VEC, CH, G><<<cgrid, 256, 0, st>>>(p, chunk_beg, chunk_end, chunk_row, n_chunks, pm, pl, pacc);
+      gat_chunk_kernel<T, VEC, CH, G, E><<<cgrid, 256, 0, st>>>(p, chunk_beg, chunk_end, chunk_row, n_chunks, pm, pl, pacc);
       GMLM_LAUNCH_CHECK();
       gat_final_kernel<T><<<unsigned(n_hub), 256, 0, st>>>(hub_row, hub_chunk_ptr, n_hub, heads, head_dim, p_drop, pm, pl,
                                                            pacc, static_cast<T*>(out), ldo, m_out, l_out);
@@ -467,13 +489,25 @@ extern "C" int gmlm_gat_fused_fwd(const int32_t* rowptr, const int32_t* col, int
   return rc;
 }
 
-extern "C" int gmlm_gat_bwd_edges(const int32_t* rowptr, const int32_t* col, int64_t num_rows, const void* z, int dtype,
-                                  int64_t ldz, const void* g, int64_t ldg, const float* a_src, const float* a_dst,
-                                  const float* m_in, const float* l_in, const float* t_in, int heads, int head_dim,
+extern "C" int gmlm_gat_fused_fwd(const int32_t* rowptr, const int32_t* col, int64_t num_rows, const void* z, int dtype,
+                                  int64_t ldz, const float* a_src, const float* a_dst, int heads, int head_dim,
                                   float negative_slope, float p_drop, uint64_t seed, int32_t hub_thresh, int64_t n_hub,
                                   int64_t n_chunks, const int32_t* hub_row, const int32_t* hub_chunk_ptr,
                                   const int32_t* chunk_beg, const int32_t* chunk_end, void* ws, size_t ws_bytes,
-                                  float* alpha_eff, float* d_score, float* da_dst, void* stream) {
+                                  void* out, int64_t ldo, float* m_out, float* l_out, void* stream) {
+  return gmlm_gat_fused_fwd_eattr(rowptr, col, num_rows, z, dtype, ldz, a_src, a_dst, nullptr, heads, head_dim,
+                                  negative_slope, p_drop, seed, hub_thresh, n_hub, n_chunks, hub_row, hub_chunk_ptr,
+                                  chunk_beg, chunk_end, ws, ws_bytes, out, ldo, m_out, l_out, stream);
+}
+
+extern "C" int gmlm_gat_bwd_edges_eattr(const int32_t* rowptr, const int32_t* col, int64_t num_rows, const void* z,
+                                        int dtype, int64_t ldz, const void* g, int64_t ldg, const float* a_src,
+                                        const float* a_dst, const float* a_edge, const float* m_in, const float* l_in,
+                                        const float* t_in, int heads, int head_dim, float negative_slope, float p_drop,
+                                        uint64_t seed, int32_t hub_thresh, int64_t n_hub, int64_t n_chunks,
+                                        const int32_t* hub_row, const int32_t* hub_chunk_ptr, const int32_t* chunk_beg,
+                                        const int32_t* chunk_end, void* ws, size_t ws_bytes, float* alpha_eff,
+                                        float* d_score, float* da_dst, void* stream) {
   GMLM_REQUIRE(dtype == GMLM_F32 || dtype == GMLM_BF16, "gat_bwd_edges: dtype must be GMLM_F32 or GMLM_BF16");
   GMLM_REQUIRE(num_rows >= 0 && heads >= 1 && heads <= 32 && head_dim >= 1, "gat_bwd_edges: bad sizes (1..32 heads)");
   const int64_t hc = int64_t(heads) * head_dim;
@@ -490,20 +524,21 @@ extern "C" int gmlm_gat_bwd_edges(const int32_t* rowptr, const int32_t* col, int
   if (int rc = head_groups(heads, head_dim, aligned, "gat_bwd_edges", &hgp)) return rc;
   cudaStream_t st = as_stream(stream);
   GatParams p{rowptr, col, z, ldz, a_src, a_dst, heads, head_dim, hgp.hg, negative_slope, p_drop, seed,
-              n_hub > 0 ? hub_thresh : 0x7fffffff};
+              n_hub > 0 ? hub_thresh : 0x7fffffff, a_edge};
   Carver cv(ws);
   int32_t* chunk_row = n_hub ? cv.take<int32_t>(n_chunks) : nullptr;
   float* da_part = n_hub ? cv.take<float>(n_chunks * heads) : nullptr;
   const dim3 grid(unsigned((num_rows * 32 + 255) / 256), unsigned(hgp.n));
   const dim3 cgrid(unsigned((n_chunks * 32 + 255) / 256), unsigned(hgp.n));
-  return dispatch_gat(dtype, hc, aligned, hgp.n, [&]<typename T, int VEC, int CH, bool G>() -> int {
-    gat_bwd_rows_kernel<T, VEC, CH, G><<<grid, 256, 0, st>>>(p, num_rows, static_cast<const T*>(g), ldg, m_in, l_in, t_in,
+  const bool edge = a_edge != nullptr;
+  return dispatch_gat(dtype, hc, aligned, hgp.n, edge, [&]<typename T, int VEC, int CH, bool G, bool E>() -> int {
+    gat_bwd_rows_kernel<T, VEC, CH, G, E><<<grid, 256, 0, st>>>(p, num_rows, static_cast<const T*>(g), ldg, m_in, l_in, t_in,
                                                             alpha_eff, d_score, da_dst);
     GMLM_LAUNCH_CHECK();
     if (n_hub) {
       chunk_rows_kernel<<<unsigned(n_hub), 128, 0, st>>>(hub_row, hub_chunk_ptr, n_hub, chunk_row);
       GMLM_LAUNCH_CHECK();
-      gat_bwd_chunk_kernel<T, VEC, CH, G><<<cgrid, 256, 0, st>>>(
+      gat_bwd_chunk_kernel<T, VEC, CH, G, E><<<cgrid, 256, 0, st>>>(
           p, chunk_beg, chunk_end, chunk_row, n_chunks, static_cast<const T*>(g), ldg, m_in, l_in, t_in, alpha_eff,
           d_score, da_part);
       GMLM_LAUNCH_CHECK();
@@ -513,6 +548,18 @@ extern "C" int gmlm_gat_bwd_edges(const int32_t* rowptr, const int32_t* col, int
     }
     return GMLM_OK;
   });
+}
+
+extern "C" int gmlm_gat_bwd_edges(const int32_t* rowptr, const int32_t* col, int64_t num_rows, const void* z, int dtype,
+                                  int64_t ldz, const void* g, int64_t ldg, const float* a_src, const float* a_dst,
+                                  const float* m_in, const float* l_in, const float* t_in, int heads, int head_dim,
+                                  float negative_slope, float p_drop, uint64_t seed, int32_t hub_thresh, int64_t n_hub,
+                                  int64_t n_chunks, const int32_t* hub_row, const int32_t* hub_chunk_ptr,
+                                  const int32_t* chunk_beg, const int32_t* chunk_end, void* ws, size_t ws_bytes,
+                                  float* alpha_eff, float* d_score, float* da_dst, void* stream) {
+  return gmlm_gat_bwd_edges_eattr(rowptr, col, num_rows, z, dtype, ldz, g, ldg, a_src, a_dst, nullptr, m_in, l_in, t_in,
+                                  heads, head_dim, negative_slope, p_drop, seed, hub_thresh, n_hub, n_chunks, hub_row,
+                                  hub_chunk_ptr, chunk_beg, chunk_end, ws, ws_bytes, alpha_eff, d_score, da_dst, stream);
 }
 
 extern "C" int gmlm_gat_dropout_mask(uint64_t seed, int64_t n, float p_drop, uint8_t* keep, void* stream) {

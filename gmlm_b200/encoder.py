@@ -17,6 +17,9 @@ What changes relative to the reference body (results stay within the parity tole
 ``GATConv(dims[k], dims[k+1] // heads, heads)`` with concatenated heads and attention dropout 0 in place of
 ``rgcn1..rgcn4``; every other submodule keeps its name and code.  The four layers share one self-looped CSR
 (``get_loop_graph``); no edge types are computed.  fp32 activations only (eval mode, or autocast with fp32 results).
+``gat_edge_types=True`` gives the GAT layers the RGCN encoder's relations as edge features: ``gatK =
+GATConv(..., edge_dim=num_relations)``, fed the one-hot of the degree-bucket edge types (cached per graph), so the
+attention score of every edge carries a learned per-relation, per-head term.
 """
 from __future__ import annotations
 
@@ -81,6 +84,7 @@ def _dense_op_dtype(x: torch.Tensor) -> Optional[torch.dtype]:
 
 
 _ET_CACHE: "OrderedDict[tuple, tuple]" = OrderedDict()
+_ONEHOT_CACHE: "OrderedDict[tuple, tuple]" = OrderedDict()
 
 
 def cached_edge_type(edge_index: torch.Tensor, num_nodes: int) -> torch.Tensor:
@@ -100,15 +104,34 @@ def cached_edge_type(edge_index: torch.Tensor, num_nodes: int) -> torch.Tensor:
         return et
 
 
+def cached_edge_type_onehot(edge_type: torch.Tensor, num_relations: int) -> torch.Tensor:
+    """float32 ``[E, num_relations]`` one-hot of ``edge_type`` (the ``edge_attr`` of the typed GAT encoder), built
+    once per edge-type tensor and keyed on its identity like ``cached_edge_type``, so no encoder call allocates it."""
+    key = (_tensor_key(edge_type), int(num_relations))
+    with _LOCK:
+        hit = _ONEHOT_CACHE.get(key)
+        if hit is not None:
+            _ONEHOT_CACHE.move_to_end(key)
+            return hit[0]
+        oh = F.one_hot(edge_type.long(), num_relations).float()
+        _ONEHOT_CACHE[key] = (oh, edge_type)
+        while len(_ONEHOT_CACHE) > 4:
+            _ONEHOT_CACHE.popitem(last=False)
+        return oh
+
+
 class GraphEncoder(nn.Module):
     def __init__(self, gnn_in_channels: int, hidden_channels: int, out_dim: int, num_relations: int = 5,
                  num_bases: int = 30, dropout_rate: float = 0.3, use_checkpoint: bool = False,
-                 act_dtype: Optional[torch.dtype] = None, conv: str = "rgcn", heads: int = 8):
+                 act_dtype: Optional[torch.dtype] = None, conv: str = "rgcn", heads: int = 8,
+                 gat_edge_types: bool = False):
         super().__init__()
         h = hidden_channels
         dims = [gnn_in_channels, h, 2 * h, 4 * h, 8 * h]
         if conv not in ("rgcn", "gat"):
             raise ValueError(f"GraphEncoder: conv must be 'rgcn' or 'gat', got {conv!r}")
+        if gat_edge_types and conv != "gat":
+            raise ValueError("GraphEncoder: gat_edge_types applies to conv='gat' only")
         if conv == "gat":
             if heads < 1 or any(d % heads for d in dims[1:]):
                 raise ValueError(f"GraphEncoder: heads = {heads} must divide every GAT layer width {dims[1:]}")
@@ -117,11 +140,13 @@ class GraphEncoder(nn.Module):
                                           "not the bf16 pipeline")
         self.dims = dims
         self.conv = conv
+        self.gat_edge_types = bool(gat_edge_types)
         self.gnn_mask_token_embed = nn.Parameter(torch.zeros(1, gnn_in_channels))   # main.py:185-186
         nn.init.xavier_uniform_(self.gnn_mask_token_embed)
         for k in range(4):                                                          # main.py:189-203
             if conv == "gat":
-                setattr(self, f"gat{k+1}", GATConv(dims[k], dims[k + 1] // heads, heads=heads))
+                setattr(self, f"gat{k+1}", GATConv(dims[k], dims[k + 1] // heads, heads=heads,
+                                                   edge_dim=num_relations if gat_edge_types else None))
             else:
                 setattr(self, f"rgcn{k+1}", RGCNConv(dims[k], dims[k + 1], num_relations=num_relations,
                                                      num_bases=num_bases, out_dtype=act_dtype))
@@ -137,8 +162,8 @@ class GraphEncoder(nn.Module):
     def _block(self, k: int):
         conv, norm, drop = getattr(self, f"{self.conv}{k}"), getattr(self, f"gnorm{k}"), getattr(self, f"dropout{k}")
 
-        def run(x, graph):
-            y = conv(x, graph)
+        def run(x, graph, *edge_attr):
+            y = conv(x, graph, *edge_attr)
             if y.size(0) > 1:                       # main.py:273
                 y = norm(y, fuse_gelu=True)         # GraphNorm + exact-erf GELU in one pass
             else:
@@ -146,10 +171,10 @@ class GraphEncoder(nn.Module):
             return drop(y)
         return run
 
-    def _run(self, k, x, graph):
+    def _run(self, k, x, graph, *edge_attr):
         if self.use_checkpoint and torch.is_grad_enabled():
-            return checkpoint(self._block(k), x, graph, use_reentrant=False)
-        return self._block(k)(x, graph)
+            return checkpoint(self._block(k), x, graph, *edge_attr, use_reentrant=False)
+        return self._block(k)(x, graph, *edge_attr)
 
     def _residual(self, lin: nn.Linear, x: torch.Tensor, acc: torch.Tensor) -> torch.Tensor:
         """``acc + lin(x)`` (main.py:281-282, 294-295).  On the tcgen05 GEMM the add happens in the epilogue: the
@@ -165,22 +190,27 @@ class GraphEncoder(nn.Module):
     def get_graph_embeddings(self, x_feat: torch.Tensor, edge_index: torch.Tensor,
                              edge_type: Optional[torch.Tensor] = None, return_layers: bool = False):
         n = x_feat.size(0)
+        ea = ()                                       # the GAT layers' edge_attr, when they take edge types
         if self.conv == "gat":
-            graph = get_loop_graph(edge_index, n)     # edge_type is not used by GAT layers
+            graph = get_loop_graph(edge_index, n)     # edge_type is not used by GAT layers without gat_edge_types
+            if self.gat_edge_types:
+                if edge_type is None:
+                    edge_type = cached_edge_type(edge_index, n)
+                ea = (cached_edge_type_onehot(edge_type, self.num_relations),)
         else:
             if edge_type is None:
                 edge_type = cached_edge_type(edge_index, n)
             graph = get_rel_graph(edge_index, edge_type, n, self.num_relations)
         outs = []
-        x1 = self._run(1, x_feat, graph)
+        x1 = self._run(1, x_feat, graph, *ea)
         outs.append(x1)                              # pre-residual outputs feed the fusion (main.py:279)
         x1 = self._residual(self.residual_proj1, x_feat, x1)
-        x2 = self._run(2, x1, graph)
+        x2 = self._run(2, x1, graph, *ea)
         outs.append(x2)
         x2 = self._residual(self.residual_proj2, x1, x2)
-        x3 = self._run(3, x2, graph)
+        x3 = self._run(3, x2, graph, *ea)
         outs.append(x3)
-        x4 = self._run(4, x3, graph)
+        x4 = self._run(4, x3, graph, *ea)
         outs.append(x4)
         fused = self.multi_scale_fusion(outs)
         return (fused, outs) if return_layers else fused

@@ -31,8 +31,9 @@ class GraphedEncoderStep:
         self.autocast = bool(autocast)
         n = x.size(0)
         self.edge_index = edge_index
-        if edge_type is None and getattr(encoder, "conv", "rgcn") == "rgcn":
-            edge_type = cached_edge_type(edge_index, n)           # GAT layers take no edge types
+        typed = getattr(encoder, "conv", "rgcn") == "rgcn" or getattr(encoder, "gat_edge_types", False)
+        if edge_type is None and typed:
+            edge_type = cached_edge_type(edge_index, n)           # GAT layers take none unless gat_edge_types
         self.edge_type = edge_type
         self.static_x = x.detach().clone().requires_grad_(x_requires_grad)
         side = torch.cuda.Stream(device=x.device)

@@ -313,7 +313,19 @@ int gmlm_gemm_tn(int num_sources, const void* const* A_host, const int64_t* lda_
  *                   d_score[e,h] (gradient of the raw score) and da_dst[i,h] = sum_e d_score;  t[i,h] must hold
  *                   <g[i,h,:], out[i,h,:]>.  da_src and dz are gathers over the transposed CSR (segment_sum_f32,
  *                   gmlm_spmm_csr with one weight column per head).
- * gat_dropout_mask: keep[i] of the counter-based hash both kernels use (index = CSR position * H + head). */
+ * gat_dropout_mask: keep[i] of the counter-based hash both kernels use (index = CSR position * H + head).
+ * gat_loop_fill   : per-edge scores alpha [E_in, H] (input order) -> a_edge [nnz, H] (forward-CSR order):
+ *                   a_edge[k] = alpha[csr_src[k]] for every entry but the row's loop entry loop_csr[r], which gets
+ *                   the mean of the row's other entries, 0 without any (upstream add_self_loops(fill_value="mean")).
+ *                   One warp per row; deterministic.
+ * gat_loop_fill_bwd: d_alpha[j] = g[in2csr[j]] + g[loop_csr[in_dst[j]]] / cnt(in_dst[j]), cnt = the row's entries
+ *                   other than its loop clamped at 1; d_alpha[j] = 0 where in2csr[j] < 0 (an input self-loop).
+ *
+ * gat_fused_fwd_eattr / gat_bwd_edges_eattr: the same two passes with a per-edge score term (upstream GATConv with
+ *                   edge_dim): a_edge [nnz, H] fp32 in CSR order, self-loop entries included, enters the score as
+ *                   leaky_relu(a_src[col[e],h] + a_edge[e,h] + a_dst[i,h]) in the forward and in the backward's
+ *                   recomputed score.  Its gradient is d_score.  a_edge = NULL is exactly gat_fused_fwd /
+ *                   gat_bwd_edges, which forward to these with NULL. */
 int gmlm_gcn_edge_weights(const int32_t* rowptr, const int32_t* col, int64_t num_rows, float* dis_ws /* [rows] */,
                           float* w /* [nnz] */, void* stream);
 int gmlm_segment_sum_f32(const float* vals, const int64_t* idx, const int32_t* rowptr, int64_t num_rows,
@@ -332,7 +344,24 @@ int gmlm_gat_bwd_edges(const int32_t* rowptr, const int32_t* col, int64_t num_ro
                        int64_t n_chunks, const int32_t* hub_row, const int32_t* hub_chunk_ptr,
                        const int32_t* chunk_beg, const int32_t* chunk_end, void* ws, size_t ws_bytes,
                        float* alpha_eff, float* d_score, float* da_dst, void* stream);
+int gmlm_gat_fused_fwd_eattr(const int32_t* rowptr, const int32_t* col, int64_t num_rows, const void* z, int dtype,
+                             int64_t ldz, const float* a_src, const float* a_dst, const float* a_edge /* [nnz, H] */,
+                             int heads, int head_dim, float negative_slope, float p_drop, uint64_t seed,
+                             int32_t hub_thresh, int64_t n_hub, int64_t n_chunks, const int32_t* hub_row,
+                             const int32_t* hub_chunk_ptr, const int32_t* chunk_beg, const int32_t* chunk_end, void* ws,
+                             size_t ws_bytes, void* out, int64_t ldo, float* m_out, float* l_out, void* stream);
+int gmlm_gat_bwd_edges_eattr(const int32_t* rowptr, const int32_t* col, int64_t num_rows, const void* z, int dtype,
+                             int64_t ldz, const void* g, int64_t ldg, const float* a_src, const float* a_dst,
+                             const float* a_edge /* [nnz, H] */, const float* m_in, const float* l_in,
+                             const float* t_in, int heads, int head_dim, float negative_slope, float p_drop,
+                             uint64_t seed, int32_t hub_thresh, int64_t n_hub, int64_t n_chunks, const int32_t* hub_row,
+                             const int32_t* hub_chunk_ptr, const int32_t* chunk_beg, const int32_t* chunk_end, void* ws,
+                             size_t ws_bytes, float* alpha_eff, float* d_score, float* da_dst, void* stream);
 int gmlm_gat_dropout_mask(uint64_t seed, int64_t n, float p_drop, uint8_t* keep, void* stream);
+int gmlm_gat_loop_fill(const float* alpha, const int32_t* csr_src, const int32_t* loop_csr, const int32_t* rowptr,
+                       int64_t num_rows, int heads, float* a_edge, void* stream);
+int gmlm_gat_loop_fill_bwd(const float* g, const int32_t* in2csr, const int32_t* in_dst, const int32_t* loop_csr,
+                           const int32_t* rowptr, int64_t num_edges, int heads, float* d_alpha, void* stream);
 
 /* ---- halo pack / unpack for the destination-row partition (SURVEY §8e; the reference has no
  *      multi-GPU path) ----
