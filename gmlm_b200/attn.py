@@ -96,7 +96,8 @@ def get_loop_graph(edge_index: torch.Tensor, num_nodes: int) -> LoopGraph:
 
 
 def _with_w(csr: CSR, w: torch.Tensor) -> CSR:
-    """A shallow view of ``csr`` carrying different per-edge weights (its band plan's hub_w no longer applies)."""
+    """A shallow view of ``csr`` carrying different per-edge weights.  Its band plan's hub_w no longer applies, and
+    without hub_w the weighted aggregation runs the CSR-order hub chunks."""
     c = CSR(**{k: getattr(csr, k) for k in csr.__dataclass_fields__})
     c.w = w
     c.hub_w = None
@@ -204,35 +205,8 @@ def _gat_backward(g, z, a_src, a_dst, m, l, out, graph: LoopGraph, slope: float,
         da_src = torch.empty((a_src.size(0), heads), dtype=torch.float32, device=dev)
         _lib.check(lib.gmlm_segment_sum_f32(_ptr(d_score), _ptr(graph.t2f), _ptr(graph.bwd.rowptr), a_src.size(0),
                                             heads, _ptr(da_src), _stream(dev)), "segment_sum")
-    bwd_w = _with_w(graph.bwd, alpha_eff[graph.t2f].contiguous())
-    if dz_out is None:
-        dz = spmm(g, bwd_w, _lib.AGG_WEIGHTED)
-    else:
-        dz = _spmm_into(g, bwd_w, dz_out)
+    dz = spmm(g, _with_w(graph.bwd, alpha_eff[graph.t2f].contiguous()), _lib.AGG_WEIGHTED, out=dz_out)
     return dz, da_src, da_dst, d_score
-
-
-def _spmm_into(x: torch.Tensor, csr: CSR, out: torch.Tensor) -> torch.Tensor:
-    """Weighted ``spmm`` written into a row-major view ``out`` with its own leading dimension."""
-    lib = _lib.load()
-    if out.dim() != 2 or out.stride(1) != 1 or out.shape != (csr.num_rows, x.size(1)) or out.dtype != x.dtype:
-        raise _lib.GmlmError("gat: the dz view must be a row-major [num_rows, H*C] tensor of g's dtype")
-    dev = x.device
-    feat = int(x.size(1))
-    w_heads = int(csr.w.size(1)) if csr.w.dim() == 2 else 1
-    n_hub = int(csr.hub_row.numel()) if csr.hub_row is not None else 0
-    n_chunks = int(csr.chunk_beg.numel()) if csr.chunk_beg is not None else 0
-    n_groups = int(csr.grp_row.numel()) - 1 if csr.grp_row is not None else 0
-    mode = _lib.AGG_WEIGHTED if csr.col.numel() else _lib.AGG_SUM      # no edges: every row is zero
-    with torch.cuda.device(dev):
-        hub_ws = torch.empty(n_chunks * feat, dtype=torch.float32, device=dev) if n_hub else None
-        _lib.check(lib.gmlm_spmm_csr(_ptr(x), _dtype_code(x, "spmm_csr"), feat, _ld(x), _ptr(csr.rowptr),
-                                     _ptr(csr.col), _ptr(csr.w) if mode == _lib.AGG_WEIGHTED else None,
-                                     w_heads if mode == _lib.AGG_WEIGHTED else 1, csr.num_rows, mode, _ptr(csr.grp_row),
-                                     n_groups, csr.hub_thresh, n_hub, n_chunks, _ptr(csr.hub_row),
-                                     _ptr(csr.hub_chunk_ptr), _ptr(csr.chunk_beg), _ptr(csr.chunk_end), _ptr(hub_ws),
-                                     _ptr(out), _ld(out), _stream(dev)), "spmm_csr")
-    return out
 
 
 class _GATAggregate(torch.autograd.Function):

@@ -108,31 +108,34 @@ def _edge_type_bucket(src: torch.Tensor, deg: torch.Tensor, bounds: Sequence[int
 
 
 # ------------------------------------------------------------------------------ A5 / A14
-def _spmm_csr(x, rowptr, col, w, num_rows, mode, grp_row, hub_thresh, hub_row, hub_chunk_ptr, chunk_beg, chunk_end,
-              hub_col=None, hub_w=None, band_plan=None, out=None):
+def _spmm_csr(x: torch.Tensor, csr: CSR, mode: int, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The aggregation kernel: out[r] = reduce over row r of ``csr`` (``mode`` AGG_SUM / AGG_MEAN / AGG_WEIGHTED; the
+    weighted mode reads ``csr.w``, one column per head when 2-D, and ``csr.hub_w`` for the band-ordered hub chunks).
+    ``out``: a row-major [num_rows, F] tensor of x's dtype, any leading dimension, written in place."""
     lib = _lib.load()
     x = _rowmajor(x)
     feat = int(x.size(1))
     dev = x.device
-    n_hub = int(hub_row.numel()) if hub_row is not None else 0
-    n_chunks = int(chunk_beg.numel()) if chunk_beg is not None else 0
-    n_groups = int(grp_row.numel()) - 1 if grp_row is not None else 0
-    n_band = (int(band_plan.numel()) - n_hub - 2) // 2 if (band_plan is not None and n_hub) else 0
+    w, hub_w = (csr.w, csr.hub_w) if mode == _lib.AGG_WEIGHTED else (None, None)
+    n_hub = int(csr.hub_row.numel()) if csr.hub_row is not None else 0
+    n_chunks = int(csr.chunk_beg.numel()) if csr.chunk_beg is not None else 0
+    n_groups = int(csr.grp_row.numel()) - 1 if csr.grp_row is not None else 0
+    n_band = (int(csr.band_plan.numel()) - n_hub - 2) // 2 if (csr.band_plan is not None and n_hub) else 0
     w_heads = int(w.size(1)) if (w is not None and w.dim() == 2) else 1
-    if col.numel() == 0 and mode == _lib.AGG_WEIGHTED:
+    if csr.col.numel() == 0 and mode == _lib.AGG_WEIGHTED:
         mode, w, w_heads = _lib.AGG_SUM, None, 1          # no edges: every row is empty, the result is zeros
     with torch.cuda.device(dev):
         if out is None:
-            out = torch.empty((num_rows, feat), dtype=x.dtype, device=dev)
-        elif out.shape != (num_rows, feat) or out.dtype != x.dtype or not out.is_contiguous():
-            raise _lib.GmlmError("spmm: `out` must be a contiguous [num_rows, feat] tensor of x's dtype")
+            out = torch.empty((csr.num_rows, feat), dtype=x.dtype, device=dev)
+        elif out.dim() != 2 or out.stride(1) != 1 or out.shape != (csr.num_rows, feat) or out.dtype != x.dtype:
+            raise _lib.GmlmError("spmm: `out` must be a row-major [num_rows, feat] tensor of x's dtype")
         hub_ws = torch.empty(max(n_chunks, n_band) * feat, dtype=torch.float32, device=dev) if n_hub else None
-        _lib.check(lib.gmlm_spmm_csr_banded(_ptr(x), _dtype_code(x, "spmm_csr"), feat, _ld(x), _ptr(rowptr), _ptr(col),
-                                            _ptr(w), w_heads, num_rows, mode, _ptr(grp_row), n_groups, hub_thresh, n_hub,
-                                            n_chunks, _ptr(hub_row), _ptr(hub_chunk_ptr), _ptr(chunk_beg),
-                                            _ptr(chunk_end), n_band, _ptr(band_plan if n_band else None),
-                                            _ptr(hub_col), _ptr(hub_w), _ptr(hub_ws), _ptr(out), feat, _stream(dev)),
-                   "spmm_csr")
+        _lib.check(lib.gmlm_spmm_csr_banded(_ptr(x), _dtype_code(x, "spmm_csr"), feat, _ld(x), _ptr(csr.rowptr),
+                                            _ptr(csr.col), _ptr(w), w_heads, csr.num_rows, mode, _ptr(csr.grp_row),
+                                            n_groups, csr.hub_thresh, n_hub, n_chunks, _ptr(csr.hub_row),
+                                            _ptr(csr.hub_chunk_ptr), _ptr(csr.chunk_beg), _ptr(csr.chunk_end), n_band,
+                                            _ptr(csr.band_plan if n_band else None), _ptr(csr.hub_col), _ptr(hub_w),
+                                            _ptr(hub_ws), _ptr(out), _ld(out), _stream(dev)), "spmm_csr")
     return out
 
 
@@ -140,15 +143,16 @@ def spmm(x: torch.Tensor, csr: CSR, mode: int, out: Optional[torch.Tensor] = Non
     """out[r] = reduce over row r of csr (no autograd).  ``out`` lets the result land in a caller-owned
     buffer (e.g. NVLink-peer-visible symmetric memory for the halo exchange)."""
     _require_cuda(x, "x")
-    weighted = mode == _lib.AGG_WEIGHTED
     if out is not None:
-        return _spmm_csr(x, csr.rowptr, csr.col, csr.w if weighted else None, csr.num_rows, mode,
-                         csr.grp_row, csr.hub_thresh, csr.hub_row, csr.hub_chunk_ptr, csr.chunk_beg, csr.chunk_end,
-                         csr.hub_col, csr.hub_w if weighted else None, csr.band_plan, out=out)
-    return torch.ops.gmlm.spmm_csr(x, csr.rowptr, csr.col, csr.w if weighted else None,
-                                   csr.num_rows, mode, csr.grp_row, csr.hub_thresh, csr.hub_row, csr.hub_chunk_ptr,
-                                   csr.chunk_beg, csr.chunk_end, csr.hub_col, csr.hub_w if weighted else None,
-                                   csr.band_plan)
+        return _spmm_csr(x, csr, mode, out)
+    c, (rows, thresh) = csr_pack(csr)
+    return _spmm_op(x, c, rows, thresh, mode)
+
+
+def _spmm_csr_op(x, rowptr, col, w, num_rows, mode, grp_row, hub_thresh, hub_row, hub_chunk_ptr, chunk_beg, chunk_end,
+                 hub_col=None, hub_w=None, band_plan=None):
+    c = [rowptr, col, w, grp_row, hub_row, hub_chunk_ptr, chunk_beg, chunk_end, hub_col, hub_w, band_plan]
+    return _spmm_csr(x, _csr_unpack(c, num_rows, hub_thresh), mode)
 
 
 # ------------------------------------------------------------------------------ A7
@@ -348,7 +352,7 @@ def _soft_mask_bwd(gy, mask, beta, need_gx):
 
 _LIB.impl("degree_i32", _degree_i32, "CUDA")
 _LIB.impl("edge_type_bucket", _edge_type_bucket, "CUDA")
-_LIB.impl("spmm_csr", _spmm_csr, "CUDA")
+_LIB.impl("spmm_csr", _spmm_csr_op, "CUDA")
 _LIB.impl("colstats", _colstats, "CUDA")
 _LIB.impl("graphnorm_fwd", _graphnorm_fwd, "CUDA")
 _LIB.impl("graphnorm_bwd", _graphnorm_bwd, "CUDA")
@@ -369,22 +373,29 @@ def csr_pack(csr: CSR):
              csr.hub_col, csr.hub_w, csr.band_plan], [int(csr.num_rows), int(csr.hub_thresh)])
 
 
-def _spmm_list(x, c, rows, thresh, mode):
-    weighted = mode == _lib.AGG_WEIGHTED
-    return _spmm_csr(x, c[0], c[1], c[2] if weighted else None, rows, mode, c[3], thresh, c[4], c[5], c[6], c[7], c[8],
-                     c[9] if weighted else None, c[10])
+def _csr_unpack(c, num_rows: int, hub_thresh: int) -> CSR:
+    """The CSR of ``csr_pack``'s eleven tensors (the fields the aggregation kernel reads)."""
+    rowptr, col, w, grp_row, hub_row, hub_chunk_ptr, chunk_beg, chunk_end, hub_col, hub_w, band_plan = c
+    return CSR(rowptr=rowptr, col=col, num_rows=num_rows, w=w, hub_thresh=hub_thresh, hub_row=hub_row,
+               hub_chunk_ptr=hub_chunk_ptr, chunk_beg=chunk_beg, chunk_end=chunk_end, hub_col=hub_col, hub_w=hub_w,
+               band_plan=band_plan, grp_row=grp_row)
+
+
+def _spmm_op(x, c, rows: int, thresh: int, mode: int):
+    """``torch.ops.gmlm.spmm_csr`` on a CSR packed by ``csr_pack``."""
+    return torch.ops.gmlm.spmm_csr(x, c[0], c[1], c[2], rows, mode, c[3], thresh, *c[4:])
 
 
 def _rgcn_aggregate_impl(x, *a):
     fwd, meta = a[0:_NC], a[2 * _NC]
     rows_f, thresh_f, _, _, n_nodes, n_slots = meta
-    h = _spmm_list(x, fwd, rows_f, thresh_f, _lib.AGG_MEAN)                 # [N*S, F]
+    h = _spmm_csr(x, _csr_unpack(fwd, rows_f, thresh_f), _lib.AGG_MEAN)     # [N*S, F]
     return h.view(n_nodes, n_slots * x.size(1))
 
 
 def _plan_aggregate_impl(rows, *a):
     fwd, meta = a[0:_NC], a[2 * _NC]
-    return _spmm_list(rows, fwd, meta[0], meta[1], _lib.AGG_WEIGHTED)
+    return _spmm_csr(rows, _csr_unpack(fwd, meta[0], meta[1]), _lib.AGG_WEIGHTED)
 
 
 def _gemm_nt_op(a1, b, bias, a2, out_dtype):
@@ -519,9 +530,8 @@ def _rgcn_aggregate_backward(ctx, gh):
     if gh.dtype != ctx.x_dtype:
         gh = gh.to(ctx.x_dtype)
     feat = gh.size(1) // n_slots
-    b = ctx.bwd
-    gx = torch.ops.gmlm.spmm_csr(gh.view(n_nodes * n_slots, feat), b[0], b[1], b[2], rows_b, _lib.AGG_WEIGHTED, b[3],
-                                 thresh_b, b[4], b[5], b[6], b[7], b[8], b[9], b[10])   # A14: gather on the transposed CSR
+    # A14: gather on the transposed CSR
+    gx = _spmm_op(gh.view(n_nodes * n_slots, feat), ctx.bwd, rows_b, thresh_b, _lib.AGG_WEIGHTED)
     return (gx,) + (None,) * (2 * _NC + 1)
 
 
@@ -533,9 +543,7 @@ def _plan_aggregate_backward(ctx, g):
     g = g.contiguous()
     if g.dtype != ctx.in_dtype:
         g = g.to(ctx.in_dtype)
-    b = ctx.bwd
-    return (torch.ops.gmlm.spmm_csr(g, b[0], b[1], b[2], ctx.meta[2], _lib.AGG_WEIGHTED, b[3], ctx.meta[3], b[4], b[5],
-                                    b[6], b[7], b[8], b[9], b[10]),) + (None,) * (2 * _NC + 1)
+    return (_spmm_op(g, ctx.bwd, ctx.meta[2], ctx.meta[3], _lib.AGG_WEIGHTED),) + (None,) * (2 * _NC + 1)
 
 
 def _graphnorm_setup(ctx, inputs, output):
@@ -767,7 +775,9 @@ def basis_compose(weight: torch.Tensor, comp: Optional[torch.Tensor], root: Opti
 def basis_compose_bwd(weight: torch.Tensor, comp: Optional[torch.Tensor], dw: torch.Tensor, slot_stride: int,
                       row_stride: int, live: Sequence[int], need_weight: bool = True, need_comp: bool = True):
     """Gradients of the composition: ``dw`` = fp32 gradient of the composed weights of the populated relations in
-    the natural strided layout ``dw[s*slot_stride + i*row_stride + o]``.  Returns (dweight [B,Fi,Fo], dcomp [R,B])."""
+    the natural strided layout ``dw[s*slot_stride + i*row_stride + o]``.  Returns (dweight [B,Fi,Fo], dcomp [R,B]).
+    Shapes the kernel does not take (more than 8 populated relations, Fo or a stride not a multiple of 4) run as two
+    stock torch matmuls."""
     lib = _lib.load()
     nb, fi, fo = (int(v) for v in weight.shape)
     S = len(live)
@@ -778,6 +788,14 @@ def basis_compose_bwd(weight: torch.Tensor, comp: Optional[torch.Tensor], dw: to
         for s, r in enumerate(live):
             dweight[r] = torch.as_strided(flat, (fi, fo), (row_stride, 1), s * slot_stride)
         return dweight, None
+    if S and not (S <= 8 and fo % 4 == 0 and slot_stride % 4 == 0 and row_stride % 4 == 0):
+        dws = torch.as_strided(dw, (S, fi, fo), (slot_stride, row_stride, 1)).reshape(S, fi * fo)
+        dweight = (comp.detach().float()[list(live)].t() @ dws).view_as(weight) if need_weight else None
+        dcomp = None
+        if need_comp:
+            dcomp = torch.zeros_like(comp, dtype=torch.float32)
+            dcomp[list(live)] = dws @ weight.detach().float().view(nb, -1).t()
+        return dweight, dcomp
     w32 = weight.detach().float().contiguous()
     c32 = comp.detach().float().contiguous()
     R = int(comp.size(0))
@@ -795,8 +813,33 @@ def basis_compose_bwd(weight: torch.Tensor, comp: Optional[torch.Tensor], dw: to
     return dweight, dcomp
 
 
-def _compose_bwd_ok(weight, S):
-    return weight.size(2) % 4 == 0 and 1 <= S <= 8
+def _to(t: Optional[torch.Tensor], dtype: Optional[torch.dtype]) -> Optional[torch.Tensor]:
+    return t.to(dtype) if t is not None else None
+
+
+def _gemm_nt_runs(op: torch.dtype, out_dtype: torch.dtype, cuda: bool, stock: bool) -> bool:
+    """Whether a dense product of the RGCN layers runs on ``gemm_nt`` (tcgen05 for 16-bit operands, 3xTF32 for fp32
+    ones) rather than on stock cuBLAS.  ``gemm_nt`` cannot write bf16 from fp32 operands, so with fp32 activations and
+    a bf16 layer output the forward runs on cuBLAS while the backward's dh / dx, fp32 like the activations, run on
+    3xTF32.  ``stock`` (``RGCNConv.use_tcgen05 = False``, fp32 operands) keeps every product on cuBLAS."""
+    return op in _OPS16 or (op == torch.float32 and cuda and out_dtype == torch.float32 and not stock)
+
+
+def _dense_nt(srcs, b: torch.Tensor, out_dtype: torch.dtype, on_gemm_nt: bool, bias=None, split: int = 0):
+    """``[srcs] @ b.T (+ bias)`` in ``out_dtype`` on the engine ``_gemm_nt_runs`` chose; ``split`` > 0 returns the
+    output's columns before and after ``split`` as two tensors.  On cuBLAS every source is its own matmul over its
+    columns of ``b``, accumulated into the first in fp32."""
+    if on_gemm_nt:
+        return gemm_nt(srcs, b, bias=bias, out_dtype=out_dtype, split=split)
+    a = srcs[0]
+    if split:
+        return (a @ b[:split].t()).to(out_dtype), (a @ b[split:].t()).to(out_dtype)
+    k = a.size(1)
+    out = a @ b[:, :k].t() if bias is None else torch.addmm(bias.float(), a, b[:, :k].t())
+    for s in srcs[1:]:
+        out.addmm_(s, b[:, k:k + s.size(1)].t())
+        k += s.size(1)
+    return out.to(out_dtype)
 
 
 def _mm_f32(a: torch.Tensor, b: torch.Tensor) -> torch.Tensor:
@@ -825,11 +868,30 @@ def _ones_source(m: int, dtype: torch.dtype, dev: torch.device) -> torch.Tensor:
     return t
 
 
-def _colsum_f32(g: torch.Tensor) -> torch.Tensor:
-    """Column sums of g (a bias gradient): one pass, fp64 accumulation, fixed order."""
-    if g.dtype not in _DT:
-        g = g.float()
-    return torch.ops.gmlm.colstats(g)[0]
+def _param_grads(srcs, g: torch.Tensor, need, bias: bool, bias_col: int = 0):
+    """fp32 parameter gradients of a product ``[srcs] @ W + bias`` with output gradient ``g``: ``[s^T g for s in srcs]``
+    (None for a source not computed) and the bias gradient ``1^T g[:, bias_col:]`` (None unless ``bias``).
+
+    16-bit operands: when any of ``need`` is set, ONE tcgen05 reduction over every source, with the ones source for the
+    bias when at most three sources leave room for it.  fp32 operands: ``_mm_f32`` for each source ``need`` marks.  A
+    bias gradient the reduction did not produce is a column sum: one pass, fp64 accumulation, fixed order."""
+    grads, dbias = [None] * len(srcs), None
+    if g.dtype in _OPS16:
+        if any(need):
+            with_ones = bias and len(srcs) < 4
+            d = gemm_tn(list(srcs) + ([_ones_source(g.size(0), g.dtype, g.device)] if with_ones else []), g)
+            k = 0
+            for i, s in enumerate(srcs):
+                grads[i] = d[k:k + s.size(1)]
+                k += s.size(1)
+            if with_ones:
+                dbias = d[k, bias_col:]
+    else:
+        grads = [_mm_f32(s.t(), g) if n else None for s, n in zip(srcs, need)]
+    if bias and dbias is None:
+        gc = g[:, bias_col:]
+        dbias = torch.ops.gmlm.colstats(gc if gc.dtype in _DT else gc.float())[0]
+    return grads, dbias
 
 
 class _RGCNTransform(torch.autograd.Function):
@@ -837,7 +899,7 @@ class _RGCNTransform(torch.autograd.Function):
 
     The composed weights never exist as a torch tensor: ``basis_compose`` reads the fp32 bases once and writes the
     GEMM's B operand in both layouts; 16-bit operand types run ONE tcgen05 GEMM over the two A sources (bias in the
-    epilogue); fp32 runs on cuBLAS (TF32 cannot meet the reference's fp32 gate).  Backward: [dh | dx] = g @ [W;root]^T
+    epilogue); fp32 operands run as 3xTF32 or on cuBLAS (``_gemm_nt_runs``).  Backward: [dh | dx] = g @ [W;root]^T
     is one more launch of the same kernel with two output maps (dh lands contiguous for the transposed aggregation);
     dW = h^T g and droot = x^T g are reductions over all nodes, produced in fp32; ``basis_compose_bwd`` turns dW
     into the basis and coefficient gradients in one pass over the bases.
@@ -851,24 +913,15 @@ class _RGCNTransform(torch.autograd.Function):
         S, fi, fo = len(live), weight.size(1), weight.size(2)
         k1 = S * fi
         ctx.stock = bool(stock)       # fp32 on stock cuBLAS (A/B switch RGCNConv.use_tcgen05 = False)
-        need_bwd_w = any(ctx.needs_input_grad[:2])
-        if op_dtype in _OPS16:
-            hq, xq = _tma_rows(h, op_dtype), (_tma_rows(x, op_dtype) if root is not None else None)
-            wn, wt = basis_compose(weight, comp, root, live, op_dtype, "agg", want_n=need_bwd_w)
-            out = gemm_nt([hq] + ([xq] if xq is not None else []), wt, bias=bias, out_dtype=out_dtype)
-        elif op_dtype == torch.float32 and h.is_cuda and out_dtype == torch.float32 and not stock:
-            # fp32 activations outside autocast (the reference's eval mode, main.py:603): the same ONE GEMM, fp32
-            # operands on the tf32 tensor cores as 3xTF32 (fp32-grade accuracy)
-            hq, xq = _tma_rows(h, torch.float32), (_tma_rows(x, torch.float32) if root is not None else None)
-            wn, wt = basis_compose(weight, comp, root, live, torch.float32, "agg", want_n=True)
-            out = gemm_nt([hq] + ([xq] if xq is not None else []), wt, bias=bias, out_dtype=torch.float32)
-        else:
-            hq, xq = h.float(), (x.float() if root is not None else None)
-            wn, _ = basis_compose(weight, comp, root, live, torch.float32, "agg", want_t=False)
-            out = hq @ wn[:k1] if bias is None else torch.addmm(bias.float(), hq, wn[:k1])
-            if xq is not None:
-                out.addmm_(xq, wn[k1:])
-            out = out.to(out_dtype)
+        # fp32 activations outside autocast (the reference's eval mode, main.py:603) run the same ONE GEMM with fp32
+        # operands on the tf32 tensor cores as 3xTF32 (fp32-grade accuracy) when the output is fp32
+        nt = _gemm_nt_runs(op_dtype, out_dtype, h.is_cuda, stock)
+        srcs = [h] + ([x] if root is not None else [])
+        srcs = [_tma_rows(t, op_dtype) if nt else t.float() for t in srcs]
+        wn, wt = basis_compose(weight, comp, root, live, op_dtype, "agg",
+                               want_n=any(ctx.needs_input_grad[:2]) or not nt, want_t=nt)
+        out = _dense_nt(srcs, wt if nt else wn.t(), out_dtype, nt, bias=bias)
+        hq, xq = srcs[0], (srcs[1] if root is not None else None)
         ctx.save_for_backward(hq, xq, wn, weight, comp)
         ctx.live, ctx.k1, ctx.op = live, k1, op_dtype
         ctx.dtypes = (weight.dtype, None if comp is None else comp.dtype, None if root is None else root.dtype,
@@ -878,70 +931,31 @@ class _RGCNTransform(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         hq, xq, wn, weight, comp = ctx.saved_tensors
-        k1, live, op = ctx.k1, ctx.live, ctx.op
-        S, fi, fo = len(live), weight.size(1), weight.size(2)
-        need_h, need_x = ctx.needs_input_grad[0], ctx.needs_input_grad[1] and xq is not None
-        dh = dx = dweight = dcomp = droot = dbias = None
+        k1, live, op, needs = ctx.k1, ctx.live, ctx.op, ctx.needs_input_grad
+        fi, fo = weight.size(1), weight.size(2)
+        need_h, need_x = needs[0], needs[1] and xq is not None
+        dh = dx = dweight = dcomp = None
         gb = g if (g.dtype == op and g.is_contiguous()) else g.to(op).contiguous()
         if need_h or need_x:
-            if op in _OPS16:
-                out_dt = torch.bfloat16 if ctx.dtypes[4] == torch.bfloat16 else torch.float32
-                gq = _tma_rows(gb)
-                if need_h and need_x:
-                    dh, dx = gemm_nt(gq, wn, out_dtype=out_dt, split=k1)      # [M, Fo] x [K1+K2, Fo]^T
-                elif need_h:
-                    dh = gemm_nt(gq, wn[:k1], out_dtype=out_dt)
-                else:
-                    dx = gemm_nt(gq, wn[k1:], out_dtype=out_dt)
-            elif op == torch.float32 and gb.is_cuda and not ctx.stock:
-                gq = _tma_rows(gb)
-                if need_h and need_x:
-                    dh, dx = gemm_nt(gq, wn, out_dtype=torch.float32, split=k1)
-                elif need_h:
-                    dh = gemm_nt(gq, wn[:k1], out_dtype=torch.float32)
-                else:
-                    dx = gemm_nt(gq, wn[k1:], out_dtype=torch.float32)
+            out_dt = torch.bfloat16 if op in _OPS16 and ctx.dtypes[4] == torch.bfloat16 else torch.float32
+            nt = _gemm_nt_runs(op, out_dt, gb.is_cuda, ctx.stock)
+            if need_h and need_x:
+                dh, dx = _dense_nt([gb], wn, out_dt, nt, split=k1)             # [M, Fo] x [K1+K2, Fo]^T
+            elif need_h:
+                dh = _dense_nt([gb], wn[:k1], out_dt, nt)
             else:
-                if need_h:
-                    dh = gb @ wn[:k1].t()
-                if need_x:
-                    dx = gb @ wn[k1:].t()
-            if dh is not None and not dh.is_contiguous():
-                dh = dh.contiguous()
-            if dh is not None and dh.dtype != ctx.dtypes[4]:
-                dh = dh.to(ctx.dtypes[4])
-            if dx is not None and dx.dtype != ctx.dtypes[5]:
-                dx = dx.to(ctx.dtypes[5])
-        dwcat = None
-        k2 = xq.size(1) if xq is not None else 0
-        if op in _OPS16 and (ctx.needs_input_grad[2] or ctx.needs_input_grad[3] or ctx.needs_input_grad[4]):
-            # dW = h^T g, droot = x^T g (and dbias = 1^T g): ONE tcgen05 reduction over the sources, fp32 result
-            srcs = [hq] + ([xq] if xq is not None else [])
-            if ctx.needs_input_grad[5]:
-                srcs.append(_ones_source(gb.size(0), op, gb.device))
-            dwcat = gemm_tn(srcs, gb)
-            if ctx.needs_input_grad[5]:
-                dbias = dwcat[k1 + k2].to(ctx.dtypes[3])
-        if ctx.needs_input_grad[2] or ctx.needs_input_grad[3]:
-            dw = dwcat[:k1] if dwcat is not None else _mm_f32(hq.t(), gb)    # [S*Fi, Fo] fp32
-            if not dw.is_contiguous():
-                dw = dw.contiguous()
-            if _compose_bwd_ok(weight, S) or comp is None:
-                dweight, dcomp = basis_compose_bwd(weight, comp, dw, fi * fo, fo, live, ctx.needs_input_grad[2],
-                                                   ctx.needs_input_grad[3] and comp is not None)
-            else:                                                             # widths the kernel does not take
-                dws = dw.view(S, fi * fo)
-                cl = comp.detach().float()[list(live)]
-                dweight = (cl.t() @ dws).view_as(weight)
-                dcomp = torch.zeros_like(comp, dtype=torch.float32)
-                dcomp[list(live)] = dws @ weight.detach().float().view(weight.size(0), -1).t()
-            dweight = dweight.to(ctx.dtypes[0]) if dweight is not None else None
-            dcomp = dcomp.to(ctx.dtypes[1]) if dcomp is not None else None
-        if ctx.needs_input_grad[4] and xq is not None:
-            droot = (dwcat[k1:k1 + k2] if dwcat is not None else _mm_f32(xq.t(), gb)).contiguous().to(ctx.dtypes[2])
-        if ctx.needs_input_grad[5] and dbias is None:
-            dbias = _colsum_f32(gb).to(ctx.dtypes[3])
-        return dh, dx, dweight, dcomp, droot, dbias, None, None, None, None
+                dx = _dense_nt([gb], wn[k1:], out_dt, nt)
+            dh = _to(dh.contiguous(), ctx.dtypes[4]) if dh is not None else None
+            dx = _to(dx, ctx.dtypes[5])
+        # dW = h^T g [S*Fi, Fo], droot = x^T g and dbias = 1^T g, fp32
+        need_w = needs[2] or needs[3]
+        (dw, *dr), dbias = _param_grads([hq] + ([xq] if xq is not None else []), gb, [need_w, needs[4]], needs[5])
+        if need_w:
+            dweight, dcomp = basis_compose_bwd(weight, comp, dw.contiguous(), fi * fo, fo, live, needs[2],
+                                               needs[3] and comp is not None)
+        droot = _to(dr[0].contiguous(), ctx.dtypes[2]) if needs[4] and xq is not None else None
+        return (dh, dx, _to(dweight, ctx.dtypes[0]), _to(dcomp, ctx.dtypes[1]), droot, _to(dbias, ctx.dtypes[3]),
+                None, None, None, None)
 
 
 class _RGCNSegCompact(torch.autograd.Function):
@@ -962,9 +976,7 @@ class _RGCNSegCompact(torch.autograd.Function):
     def forward(ctx, x, weight, comp, root, bias, plan, num_nodes, live, out_dtype, op_dtype):
         live = tuple(int(v) for v in live)
         S, fi, fo = len(live), weight.size(1), weight.size(2)
-        h_c = _spmm_csr(x, plan.fwd.rowptr, plan.fwd.col, None, plan.fwd.num_rows, _lib.AGG_MEAN, plan.fwd.grp_row,
-                        plan.fwd.hub_thresh, plan.fwd.hub_row, plan.fwd.hub_chunk_ptr, plan.fwd.chunk_beg,
-                        plan.fwd.chunk_end, plan.fwd.hub_col, None, plan.fwd.band_plan)
+        h_c = _spmm_csr(x, plan.fwd, _lib.AGG_MEAN)
         hq = _tma_rows(h_c, op_dtype)
         xq = _tma_rows(x[:num_nodes], op_dtype)
         wn, wt = basis_compose(weight, comp, root, live, op_dtype, "agg")
@@ -989,7 +1001,7 @@ class _RGCNSegCompact(torch.autograd.Function):
         g = g.contiguous()
         gq = _tma_rows(g, op)
         acc_dt = torch.bfloat16 if ctx.dtypes[4] == torch.bfloat16 else torch.float32
-        dx = dweight = dcomp = droot = dbias = None
+        dx = dweight = dcomp = None
         need_x = ctx.needs_input_grad[0]
         need_w = ctx.needs_input_grad[1] or ctx.needs_input_grad[2]
         g_src = g if g.dtype in _DT else g.float()                         # the row gather takes fp32 / bf16
@@ -1011,40 +1023,25 @@ class _RGCNSegCompact(torch.autograd.Function):
             rows_done = a + c + pad
         if need_x:
             dh_c = torch.cat(dh_parts, dim=0) if dh_parts else torch.zeros((0, fi), dtype=acc_dt, device=g.device)
-            b = plan.bwd
             if dh_c.size(0) == 0:                                                         # a graph without edges
                 dx = torch.zeros((ctx.num_src, fi), dtype=acc_dt, device=g.device)
             else:
-                dx = _spmm_csr(dh_c, b.rowptr, b.col, b.w, b.num_rows, _lib.AGG_WEIGHTED, b.grp_row, b.hub_thresh,
-                               b.hub_row, b.hub_chunk_ptr, b.chunk_beg, b.chunk_end, b.hub_col, b.hub_w,
-                               b.band_plan)                                              # [num_src, Fi]
+                dx = _spmm_csr(dh_c, plan.bwd, _lib.AGG_WEIGHTED)                         # [num_src, Fi]
             dxr = gemm_nt(gq, wn[S * fi:], out_dtype=acc_dt)                              # root term, local rows
             if dx.size(0) == dxr.size(0):
                 dx = dx + dxr
             else:
                 dx[:n] += dxr
-            if dx.dtype != ctx.dtypes[4]:
-                dx = dx.to(ctx.dtypes[4])
-        if ctx.needs_input_grad[3] or ctx.needs_input_grad[4]:
-            srcs = [xq] + ([_ones_source(gq.size(0), op, gq.device)] if ctx.needs_input_grad[4] else [])
-            d = gemm_tn(srcs, gq)
-            if ctx.needs_input_grad[3]:
-                droot = d[:fi].contiguous().to(ctx.dtypes[2])
-            if ctx.needs_input_grad[4]:
-                dbias = d[fi].to(ctx.dtypes[3])
+            dx = dx.to(ctx.dtypes[4])
+        # [droot; dbias] = [x | 1]^T g in one reduction, also when only the bias needs it
+        (droot,), dbias = _param_grads([xq], gq, [ctx.needs_input_grad[3] or ctx.needs_input_grad[4]],
+                                       ctx.needs_input_grad[4])
+        droot = _to(droot.contiguous(), ctx.dtypes[2]) if ctx.needs_input_grad[3] else None
         if need_w:
-            if _compose_bwd_ok(weight, S) or comp is None:
-                dweight, dcomp = basis_compose_bwd(weight, comp, dw, fi * fo, fo, live, ctx.needs_input_grad[1],
-                                                   ctx.needs_input_grad[2] and comp is not None)
-            else:
-                dws = dw.view(S, fi * fo)
-                cl = comp.detach().float()[list(live)]
-                dweight = (cl.t() @ dws).view_as(weight)
-                dcomp = torch.zeros_like(comp, dtype=torch.float32)
-                dcomp[list(live)] = dws @ weight.detach().float().view(weight.size(0), -1).t()
-            dweight = dweight.to(ctx.dtypes[0]) if dweight is not None else None
-            dcomp = dcomp.to(ctx.dtypes[1]) if dcomp is not None else None
-        return dx, dweight, dcomp, droot, dbias, None, None, None, None, None
+            dweight, dcomp = basis_compose_bwd(weight, comp, dw, fi * fo, fo, live, ctx.needs_input_grad[1],
+                                               ctx.needs_input_grad[2] and comp is not None)
+        return (dx, _to(dweight, ctx.dtypes[0]), _to(dcomp, ctx.dtypes[1]), droot, _to(dbias, ctx.dtypes[3]),
+                None, None, None, None, None)
 
 
 def rgcn_segment_compact(x: torch.Tensor, graph: RelGraph, weight: torch.Tensor, comp: Optional[torch.Tensor],
@@ -1074,14 +1071,11 @@ class _RGCNTransformFirst(torch.autograd.Function):
         if bias is not None:
             bias_cat = torch.cat([bias.new_zeros(S * fo), bias.detach()]).float()
         ctx.stock = bool(stock)
-        if op_dtype in _OPS16 or (op_dtype == torch.float32 and out_dtype == torch.float32 and not stock):
-            xq = _tma_rows(x, op_dtype)                   # fp32 operands: 3xTF32 (the reference's eval mode)
-            wn, wt = basis_compose(weight, comp, root, live, op_dtype, "tf", want_n=ctx.needs_input_grad[0])
-            z = gemm_nt(xq, wt, bias=bias_cat, out_dtype=out_dtype)
-        else:
-            xq = x.float()
-            wn, _ = basis_compose(weight, comp, root, live, torch.float32, "tf", want_t=False)
-            z = (xq @ wn if bias_cat is None else torch.addmm(bias_cat, xq, wn)).to(out_dtype)
+        nt = _gemm_nt_runs(op_dtype, out_dtype, x.is_cuda, stock)
+        xq = _tma_rows(x, op_dtype) if nt else x.float()
+        wn, wt = basis_compose(weight, comp, root, live, op_dtype, "tf", want_n=ctx.needs_input_grad[0] or not nt,
+                               want_t=nt)
+        z = _dense_nt([xq], wt if nt else wn.t(), out_dtype, nt, bias=bias_cat)
         ctx.save_for_backward(xq, wn, weight, comp)
         ctx.live, ctx.op = live, op_dtype
         ctx.dtypes = (weight.dtype, None if comp is None else comp.dtype, root.dtype,
@@ -1091,47 +1085,24 @@ class _RGCNTransformFirst(torch.autograd.Function):
     @staticmethod
     def backward(ctx, gz):
         xq, wn, weight, comp = ctx.saved_tensors
-        live, op = ctx.live, ctx.op
-        S, fi, fo = len(live), weight.size(1), weight.size(2)
-        dx = dweight = dcomp = droot = dbias = None
+        live, op, needs = ctx.live, ctx.op, ctx.needs_input_grad
+        S, fo = len(live), weight.size(2)
+        dx = dweight = dcomp = droot = None
         gb = gz if (gz.dtype == op and gz.is_contiguous()) else gz.to(op).contiguous()
-        if ctx.needs_input_grad[0]:
-            if op in _OPS16 or (op == torch.float32 and gb.is_cuda and not ctx.stock):
-                dx = gemm_nt(_tma_rows(gb), wn, out_dtype=torch.bfloat16 if ctx.dtypes[4] == torch.bfloat16 else torch.float32)
-                if not dx.is_contiguous():
-                    dx = dx.contiguous()
-            else:
-                dx = gb @ wn.t()
-            if dx.dtype != ctx.dtypes[4]:
-                dx = dx.to(ctx.dtypes[4])
-        if any(ctx.needs_input_grad[1:4]):
-            if op in _OPS16:                                                  # [Fi, (S+1)*Fo] fp32 (+ 1^T g rows)
-                dwn = gemm_tn([xq] + ([_ones_source(gb.size(0), op, gb.device)] if ctx.needs_input_grad[4] else []), gb)
-                if ctx.needs_input_grad[4]:
-                    dbias = dwn[fi, S * fo:].to(ctx.dtypes[3])
-                dwn = dwn[:fi]
-            else:
-                dwn = _mm_f32(xq.t(), gb)
-            if not dwn.is_contiguous():
-                dwn = dwn.contiguous()
-            ld = dwn.size(1)
-            if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
-                if (_compose_bwd_ok(weight, S) and ld % 4 == 0) or comp is None:
-                    dweight, dcomp = basis_compose_bwd(weight, comp, dwn, fo, ld, live, ctx.needs_input_grad[1],
-                                                       ctx.needs_input_grad[2] and comp is not None)
-                else:
-                    dws = dwn[:, :S * fo].reshape(fi, S, fo).permute(1, 0, 2).reshape(S, fi * fo)
-                    cl = comp.detach().float()[list(live)]
-                    dweight = (cl.t() @ dws).view_as(weight)
-                    dcomp = torch.zeros_like(comp, dtype=torch.float32)
-                    dcomp[list(live)] = dws @ weight.detach().float().view(weight.size(0), -1).t()
-                dweight = dweight.to(ctx.dtypes[0]) if dweight is not None else None
-                dcomp = dcomp.to(ctx.dtypes[1]) if dcomp is not None else None
-            if ctx.needs_input_grad[3]:
-                droot = dwn[:, S * fo:].contiguous().to(ctx.dtypes[2])
-        if ctx.needs_input_grad[4] and dbias is None:
-            dbias = _colsum_f32(gb[:, S * fo:]).to(ctx.dtypes[3])
-        return dx, dweight, dcomp, droot, dbias, None, None, None, None
+        if needs[0]:
+            out_dt = torch.bfloat16 if op in _OPS16 and ctx.dtypes[4] == torch.bfloat16 else torch.float32
+            dx = _to(_dense_nt([gb], wn, out_dt, _gemm_nt_runs(op, out_dt, gb.is_cuda, ctx.stock)).contiguous(),
+                     ctx.dtypes[4])
+        # dWn = x^T dZ [Fi, (S+1)*Fo] fp32; the bias is on the root slab only
+        (dwn,), dbias = _param_grads([xq], gb, [any(needs[1:4])], needs[4], bias_col=S * fo)
+        if needs[1] or needs[2]:
+            dwn = dwn.contiguous()
+            dweight, dcomp = basis_compose_bwd(weight, comp, dwn, fo, dwn.size(1), live, needs[1],
+                                               needs[2] and comp is not None)
+        if needs[3]:
+            droot = _to(dwn[:, S * fo:].contiguous(), ctx.dtypes[2])
+        return (dx, _to(dweight, ctx.dtypes[0]), _to(dcomp, ctx.dtypes[1]), droot, _to(dbias, ctx.dtypes[3]),
+                None, None, None, None)
 
 
 class _LinearNT(torch.autograd.Function):
@@ -1156,7 +1127,7 @@ class _LinearNT(torch.autograd.Function):
         wtq, *xq = ctx.saved_tensors
         op = ctx.op
         gb = g if (g.dtype == op and g.is_contiguous()) else g.to(op).contiguous()
-        dwt = dbias = dadd = None
+        dwt = dadd = None
         dxs = [None] * len(xq)
         if any(ctx.needs_input_grad[5:]):
             all_bf16 = all(d == torch.bfloat16 for d in ctx.dtypes[2])
@@ -1175,20 +1146,14 @@ class _LinearNT(torch.autograd.Function):
                     k0 += v
             for i, d in enumerate(parts):
                 if ctx.needs_input_grad[5 + i]:
-                    dxs[i] = d if d.dtype == ctx.dtypes[2][i] else d.to(ctx.dtypes[2][i])
+                    dxs[i] = d.to(ctx.dtypes[2][i])
+        # dWt = g^T [x_0 | x_1 | ..] as ([x..]^T g)^T: one tcgen05 reduction over the sources (+ 1^T g = dbias)
+        dws, dbias = _param_grads(xq, gb, [ctx.needs_input_grad[0]] * len(xq), ctx.needs_input_grad[1])
         if ctx.needs_input_grad[0]:
-            # dWt = g^T [x_0 | x_1 | ..] as ([x..]^T g)^T: one tcgen05 reduction over the sources (+ 1^T g = dbias)
-            with_bias = ctx.needs_input_grad[1] and len(xq) < 4
-            d = gemm_tn(list(xq) + ([_ones_source(gb.size(0), op, gb.device)] if with_bias else []), gb)
-            kx = sum(int(x.size(1)) for x in xq)
-            if with_bias:
-                dbias = d[kx].to(ctx.dtypes[1])
-            dwt = d[:kx].t().contiguous().to(ctx.dtypes[0])
-        if ctx.needs_input_grad[1] and dbias is None:
-            dbias = _colsum_f32(gb).to(ctx.dtypes[1])
+            dwt = torch.cat([d.t() for d in dws], dim=1).to(ctx.dtypes[0])
         if ctx.needs_input_grad[2]:
             dadd = g
-        return (dwt, dbias, dadd, None, None, *dxs)
+        return (dwt, _to(dbias, ctx.dtypes[1]), dadd, None, None, *dxs)
 
 
 def linear_nt(x, wt: torch.Tensor, bias: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None,
@@ -1235,7 +1200,8 @@ def rgcn_transform_first(x: torch.Tensor, graph: RelGraph, weight: torch.Tensor,
         z = _RGCNTransformFirst.apply(x, weight, comp, root, bias, tuple(live), z_dt, op, not use_tcgen05)
         fl, fm = csr_pack(fplan)
         bl, bm = csr_pack(bplan)
-        out = torch.ops.gmlm.plan_aggregate(z.view(graph.num_src * (S + 1), fo), *fl, *bl, fm + bm)
+        # one Fo-wide row per (node, slab); a GEMM output whose row pitch is padded to 16 bytes is copied first
+        out = torch.ops.gmlm.plan_aggregate(z.reshape(graph.num_src * (S + 1), fo), *fl, *bl, fm + bm)
     return out if out.dtype == out_dt else out.to(out_dt)
 
 

@@ -42,7 +42,7 @@ def test_compose_forward_without_bases_or_root(cuda_dev):
     assert torch.equal(wn, weight[[0, 2, 3]].reshape(-1, 40)) and torch.equal(wt, wn.t())
 
 
-@pytest.mark.parametrize("fi,fo", [(64, 64), (300, 512), (257, 36), (2048, 256)])
+@pytest.mark.parametrize("fi,fo", [(64, 64), (300, 512), (257, 36), (2048, 256), (100, 7), (33, 22)])
 @pytest.mark.parametrize("live", [(0, 1, 2, 3), (2,)])
 @pytest.mark.parametrize("layout", ["agg", "tf"])
 def test_compose_backward_matches_autograd(cuda_dev, fi, fo, live, layout):

@@ -52,7 +52,8 @@ def test_dst_plan_matches_numpy_restatement(cuda_dev):
     assert torch.equal(dense_t, dense.t().contiguous())
 
 
-@pytest.mark.parametrize("n,e,fi,fo", [(183, 300, 1703, 64), (3000, 40000, 256, 64), (500, 6000, 96, 32), (1, 2, 16, 8)])
+@pytest.mark.parametrize("n,e,fi,fo", [(183, 300, 1703, 64), (3000, 40000, 256, 64), (500, 6000, 96, 32),
+                                      (500, 6000, 96, 22), (1, 2, 16, 8)])
 def test_transform_first_fp32_matches_oracle_and_aggregate_first(cuda_dev, n, e, fi, fo):
     torch.manual_seed(1)
     ei = synth.rmat_edges(n, e, seed=n) if n > 1 else torch.zeros(2, e, dtype=torch.int64)
@@ -141,7 +142,8 @@ def test_transform_first_on_a_partition_shaped_graph(cuda_dev):
 
 
 @pytest.mark.parametrize("mode", ["autocast", "bf16"])
-@pytest.mark.parametrize("n,e,fi,fo", [(3000, 4500, 300, 512), (2000, 9000, 64, 128), (500, 200, 128, 256), (64, 0, 64, 64)])
+@pytest.mark.parametrize("n,e,fi,fo", [(3000, 4500, 300, 512), (2000, 9000, 64, 128), (500, 200, 128, 256),
+                                      (2000, 9000, 64, 22), (64, 0, 64, 64)])
 def test_segment_compact_matches_dense_and_oracle(cuda_dev, mode, n, e, fi, fo):
     """The segment-compact formulation (one GEMM per populated relation over the non-empty (dst, rel) segments only,
     RelGraph.seg_plan) against the dense aggregate-first layer and the fp64 oracle: output, input gradient and every
