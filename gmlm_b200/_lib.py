@@ -34,10 +34,12 @@ SIGNATURES = {
     "gmlm_dst_plan": (_int, [_p, _p, _i64, _int, _i64, _i64, _p, _p, _p, _p, _p]),
     "gmlm_hub_count": (_int, [_p, _i64, _i32, C.POINTER(_i64), _p, _sz, _p]),
     "gmlm_hub_fill": (_int, [_p, _i64, _i32, _i64, _i64, _p, _p, _p, _p, _p, _sz, _p]),
+    "gmlm_col_rank_workspace_bytes": (_sz, [_i64]),
+    "gmlm_col_rank": (_int, [_p, _i64, _i64, _p, _p, _sz, _p]),
     "gmlm_hub_band_workspace_bytes": (_sz, [_i64]),
-    "gmlm_hub_band_sort": (_int, [_p, _p, _p, _i64, _p, _p, _i64, _int, _i32, _i32, _p, _p, _p, C.POINTER(_i64), _p,
-                                  _sz, _p]),
-    "gmlm_hub_band_order": (_int, [_p, _p, _i64, _i64, _i64, _int, _i32, _i32, _p, _p, _sz, _p]),
+    "gmlm_hub_band_sort": (_int, [_p, _p, _p, _p, _i64, _p, _p, _i64, _int, _i32, _i32, _p, _p, _p, C.POINTER(_i64),
+                                  _p, _sz, _p]),
+    "gmlm_hub_band_order": (_int, [_p, _p, _p, _i64, _i64, _i64, _int, _i32, _i32, _p, _p, _sz, _p]),
     "gmlm_group_plan_size": (_i64, [_i64, _i64, _i64]),
     "gmlm_group_plan": (_int, [_p, _i64, _i64, _i64, _p, _p]),
     "gmlm_spmm_csr": (_int, [_p, _int, _i64, _i64, _p, _p, _p, _i32, _i64, _int, _p, _i64, _i32, _i64, _i64, _p, _p,

@@ -289,17 +289,47 @@ __global__ void hub_fill_chunks_kernel(const int32_t* __restrict__ rowptr, const
   }
 }
 
+// ------------------------------------------------------------------ use rank of gathered rows
+// count[c] = edges of the CSR that gather row c (integer atomics: order-independent)
+__global__ void col_count_kernel(const int32_t* __restrict__ col, int64_t nnz, int64_t num_cols,
+                                 int32_t* __restrict__ count, int* __restrict__ err) {
+  for (int64_t e = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; e < nnz; e += int64_t(gridDim.x) * blockDim.x) {
+    const int32_t c = col[e];
+    if (c >= 0 && c < num_cols) atomicAdd(count + c, 1);
+    else flag_error(err);
+  }
+}
+
+// In place: count -> sort key nnz - count (the stable ascending sort then orders by count desc, id asc); vals = id.
+__global__ void col_rank_keys_kernel(uint32_t* __restrict__ keys, int64_t nnz, int64_t num_cols,
+                                     int32_t* __restrict__ vals) {
+  for (int64_t c = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; c < num_cols; c += int64_t(gridDim.x) * blockDim.x) {
+    keys[c] = uint32_t(nnz - int64_t(keys[c]));
+    vals[c] = int32_t(c);
+  }
+}
+
+__global__ void col_rank_scatter_kernel(const int32_t* __restrict__ order, int64_t num_cols, int32_t* __restrict__ rank) {
+  for (int64_t r = blockIdx.x * int64_t(blockDim.x) + threadIdx.x; r < num_cols; r += int64_t(gridDim.x) * blockDim.x)
+    rank[order[r]] = int32_t(r);
+}
+
 // ------------------------------------------------------------------ band-ordered hub plan
-// The hub edges listed row by row (hub_off[h] = first position of hub row h): key = gathered row, value = position.
+// The band key of a gathered row: its use rank when a rank is given, else the row id itself.
+__device__ __forceinline__ int32_t band_key(const int32_t* __restrict__ rank, int32_t c) { return rank ? rank[c] : c; }
+
+// The hub edges listed row by row (hub_off[h] = first position of hub row h): key = band key of the gathered row,
+// value = position.
 __global__ void hub_band_keys_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ col,
-                                     const int32_t* __restrict__ hub_row, const int32_t* __restrict__ hub_off,
-                                     int64_t n_hub, uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
+                                     const int32_t* __restrict__ rank, const int32_t* __restrict__ hub_row,
+                                     const int32_t* __restrict__ hub_off, int64_t n_hub, uint32_t* __restrict__ keys,
+                                     int32_t* __restrict__ vals) {
   const int64_t h = (blockIdx.x * int64_t(blockDim.x) + threadIdx.x) >> 5;
   const int lane = threadIdx.x & 31;
   if (h >= n_hub) return;
   const int32_t e0 = rowptr[hub_row[h]], o0 = hub_off[h], n = hub_off[h + 1] - o0;
   for (int32_t j = lane; j < n; j += 32) {
-    keys[o0 + j] = uint32_t(col[e0 + j]);
+    keys[o0 + j] = uint32_t(band_key(rank, col[e0 + j]));
     vals[o0 + j] = o0 + j;
   }
 }
@@ -331,19 +361,19 @@ __global__ void hub_band_gather_kernel(const uint32_t* __restrict__ row_key, con
   }
 }
 
-// Chunk starts of one hub row, whose edges [a, b) of hub_col are sorted by source.  A band boundary (the source
+// Chunk starts of one hub row, whose edges [a, b) of hub_col are sorted by band key.  A band boundary (the key
 // crosses a multiple of 2^shift) is kept as a cut when the pieces on both sides hold at least `min_run` edges; every
 // piece between kept cuts is then cut into chunks of `thresh` edges.  emit(k, start) receives the k-th chunk start.
 template <typename F>
-__device__ int32_t hub_band_walk(const int32_t* __restrict__ hub_col, int32_t a, int32_t b, int shift, int32_t thresh,
-                                 int32_t min_run, F emit) {
+__device__ int32_t hub_band_walk(const int32_t* __restrict__ hub_col, const int32_t* __restrict__ rank, int32_t a,
+                                 int32_t b, int shift, int32_t thresh, int32_t min_run, F emit) {
   int32_t k = 0, last = a, s = a;
   while (s < b) {
-    const int64_t next = (int64_t(hub_col[s] >> shift) + 1) << shift;   // first source of the next band
-    int32_t lo = s, hi = b;                                              // first p in (s, b] with hub_col[p] >= next
+    const int64_t next = (int64_t(band_key(rank, hub_col[s]) >> shift) + 1) << shift;   // first key of the next band
+    int32_t lo = s, hi = b;                                              // first p in (s, b] with key(p) >= next
     while (lo < hi) {
       const int32_t mid = lo + ((hi - lo) >> 1);
-      if (int64_t(hub_col[mid]) >= next) hi = mid; else lo = mid + 1;
+      if (int64_t(band_key(rank, hub_col[mid])) >= next) hi = mid; else lo = mid + 1;
     }
     const int32_t p = lo;
     if (p < b && (p - last < min_run || b - p < min_run)) { s = p; continue; }
@@ -353,25 +383,26 @@ __device__ int32_t hub_band_walk(const int32_t* __restrict__ hub_col, int32_t a,
   return k;
 }
 
-__global__ void hub_band_count_kernel(const int32_t* __restrict__ hub_col, const int32_t* __restrict__ hub_off,
-                                      int64_t n_hub, int shift, int32_t thresh, int32_t min_run,
-                                      int32_t* __restrict__ nch /* [n_hub+1] */) {
+__global__ void hub_band_count_kernel(const int32_t* __restrict__ hub_col, const int32_t* __restrict__ rank,
+                                      const int32_t* __restrict__ hub_off, int64_t n_hub, int shift, int32_t thresh,
+                                      int32_t min_run, int32_t* __restrict__ nch /* [n_hub+1] */) {
   const int64_t h = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
-  if (h < n_hub) nch[h] = hub_band_walk(hub_col, hub_off[h], hub_off[h + 1], shift, thresh, min_run, [](int32_t, int32_t) {});
+  if (h < n_hub)
+    nch[h] = hub_band_walk(hub_col, rank, hub_off[h], hub_off[h + 1], shift, thresh, min_run, [](int32_t, int32_t) {});
   else if (h == n_hub) nch[h] = 0;
 }
 
-__global__ void hub_band_fill_kernel(const int32_t* __restrict__ hub_col, const int32_t* __restrict__ hub_off,
-                                     const int32_t* __restrict__ band_chunk_ptr, int64_t n_hub, int shift,
-                                     int32_t thresh, int32_t min_run, int32_t* __restrict__ cut, uint32_t* __restrict__ keys,
-                                     int32_t* __restrict__ vals) {
+__global__ void hub_band_fill_kernel(const int32_t* __restrict__ hub_col, const int32_t* __restrict__ rank,
+                                     const int32_t* __restrict__ hub_off, const int32_t* __restrict__ band_chunk_ptr,
+                                     int64_t n_hub, int shift, int32_t thresh, int32_t min_run, int32_t* __restrict__ cut,
+                                     uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
   const int64_t h = blockIdx.x * int64_t(blockDim.x) + threadIdx.x;
   if (h == n_hub) cut[band_chunk_ptr[n_hub]] = hub_off[n_hub];        // the end of the last chunk
   if (h >= n_hub) return;
   const int32_t c0 = band_chunk_ptr[h];
-  hub_band_walk(hub_col, hub_off[h], hub_off[h + 1], shift, thresh, min_run, [&](int32_t k, int32_t q) {
+  hub_band_walk(hub_col, rank, hub_off[h], hub_off[h + 1], shift, thresh, min_run, [&](int32_t k, int32_t q) {
     cut[c0 + k] = q;
-    keys[c0 + k] = uint32_t(hub_col[q] >> shift);                     // band of the chunk's first edge
+    keys[c0 + k] = uint32_t(band_key(rank, hub_col[q]) >> shift);     // band of the chunk's first edge
     vals[c0 + k] = c0 + k;
   });
 }
@@ -651,14 +682,58 @@ int gmlm_hub_fill(const int32_t* rowptr, int64_t num_rows, int32_t thresh, int64
   return GMLM_OK;
 }
 
+size_t gmlm_col_rank_workspace_bytes(int64_t num_cols) {
+  if (num_cols < 1) num_cols = 1;
+  // keys, sorted keys (u32), ids, order (i32) + the per-call error flag + alignment slack
+  return sort_temp_bytes(num_cols) + 4 * (size_t(num_cols) * 4 + 256) + 4096;
+}
+
+int gmlm_col_rank(const int32_t* col, int64_t nnz, int64_t num_cols, int32_t* rank, void* ws, size_t ws_bytes,
+                  void* stream) {
+  GMLM_REQUIRE(nnz >= 0 && num_cols >= 0 && nnz < (int64_t(1) << 31) - 1 && num_cols < (int64_t(1) << 31) - 1,
+               "col_rank: bad sizes");
+  GMLM_REQUIRE(ws_bytes >= gmlm_col_rank_workspace_bytes(num_cols), "col_rank: workspace too small");
+  if (num_cols == 0) return GMLM_OK;
+  GMLM_REQUIRE(rank && (nnz == 0 || col), "col_rank: null pointer");
+  cudaStream_t st = as_stream(stream);
+  Carver cv(ws);
+  uint32_t* keys_a = cv.take<uint32_t>(num_cols);
+  uint32_t* keys_b = cv.take<uint32_t>(num_cols);
+  int32_t* vals_a = cv.take<int32_t>(num_cols);
+  int32_t* order = cv.take<int32_t>(num_cols);
+  int* d_flag = cv.take<int>(1);
+  void* prim_ws = cv.take<char>(0);
+  const size_t prim_bytes = ws_bytes - cv.used();
+  GMLM_CUDA_TRY(cudaMemsetAsync(d_flag, 0, sizeof(int), st));
+  GMLM_CUDA_TRY(cudaMemsetAsync(keys_a, 0, size_t(num_cols) * sizeof(uint32_t), st));
+  if (nnz > 0) {
+    col_count_kernel<<<grid_for(nnz, 4), kThreads, 0, st>>>(col, nnz, num_cols, reinterpret_cast<int32_t*>(keys_a),
+                                                            d_flag);
+    GMLM_LAUNCH_CHECK();
+  }
+  col_rank_keys_kernel<<<grid_for(num_cols, 2), kThreads, 0, st>>>(keys_a, nnz, num_cols, vals_a);
+  GMLM_LAUNCH_CHECK();
+  // stable: rows of equal use keep ascending id order
+  if (int rc = prim::radix_sort_pairs(keys_a, vals_a, keys_b, order, num_cols, bits_for(uint64_t(nnz) + 1), prim_ws,
+                                      prim_bytes, st))
+    return rc;
+  col_rank_scatter_kernel<<<grid_for(num_cols, 2), kThreads, 0, st>>>(order, num_cols, rank);
+  GMLM_LAUNCH_CHECK();
+  int flag = 0;
+  if (int rc = read_flag(d_flag, st, &flag)) return rc;
+  if (flag) return fail(GMLM_ERR_INDEX, "col_rank: col outside [0,%lld)", (long long)num_cols);
+  return GMLM_OK;
+}
+
 size_t gmlm_hub_band_workspace_bytes(int64_t n_hub_edges) {
   if (n_hub_edges < 1) n_hub_edges = 1;
   const size_t prim_bytes = std::max(sort_temp_bytes(n_hub_edges), scan_temp_bytes(n_hub_edges + 1));
   return prim_bytes + 4 * (size_t(n_hub_edges) * 4 + 256) + 4096;
 }
 
-int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w, int64_t n_hub, const int32_t* hub_row,
-                       const int32_t* hub_off, int64_t n_hub_edges, int band_shift, int32_t thresh, int32_t min_run,
+int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w, const int32_t* rank, int64_t n_hub,
+                       const int32_t* hub_row, const int32_t* hub_off, int64_t n_hub_edges, int band_shift,
+                       int32_t thresh, int32_t min_run,
                        int32_t* hub_col, float* hub_w, int32_t* band_chunk_ptr, int64_t* n_band_host, void* ws,
                        size_t ws_bytes, void* stream) {
   GMLM_REQUIRE(n_hub >= 0 && n_hub_edges >= 0 && n_hub_edges < (int64_t(1) << 31) - 1, "hub_band_sort: bad sizes");
@@ -676,9 +751,9 @@ int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w
   int32_t* vals_b = cv.take<int32_t>(n_hub_edges);
   void* prim_ws = cv.take<char>(0);
   const size_t prim_bytes = ws_bytes - cv.used();
-  // stable by source, then stable by hub row: each row's edges in source order, ties in CSR order
-  hub_band_keys_kernel<<<int((n_hub * 32 + kThreads - 1) / kThreads), kThreads, 0, st>>>(rowptr, col, hub_row, hub_off,
-                                                                                       n_hub, keys_a, vals_a);
+  // stable by band key, then stable by hub row: each row's edges in key order, ties in CSR order
+  hub_band_keys_kernel<<<int((n_hub * 32 + kThreads - 1) / kThreads), kThreads, 0, st>>>(rowptr, col, rank, hub_row,
+                                                                                       hub_off, n_hub, keys_a, vals_a);
   GMLM_LAUNCH_CHECK();
   if (int rc = prim::radix_sort_pairs(keys_a, vals_a, keys_b, vals_b, n_hub_edges, 31, prim_ws, prim_bytes, st)) return rc;
   hub_band_rowkey_kernel<<<grid_for(n_hub_edges, 2), kThreads, 0, st>>>(vals_b, n_hub_edges, hub_off, n_hub, keys_b);
@@ -690,7 +765,7 @@ int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w
                                                                         hub_off, col, w, hub_col, hub_w);
   GMLM_LAUNCH_CHECK();
   hub_band_count_kernel<<<int((n_hub + 1 + kThreads - 1) / kThreads), kThreads, 0, st>>>(
-      hub_col, hub_off, n_hub, band_shift, thresh, min_run, band_chunk_ptr);
+      hub_col, rank, hub_off, n_hub, band_shift, thresh, min_run, band_chunk_ptr);
   GMLM_LAUNCH_CHECK();
   if (int rc = prim::exclusive_scan_i32(band_chunk_ptr, band_chunk_ptr, n_hub + 1, prim_ws, prim_bytes, st)) return rc;
   int32_t n_band = 0;
@@ -700,9 +775,9 @@ int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w
   return GMLM_OK;
 }
 
-int gmlm_hub_band_order(const int32_t* hub_col, const int32_t* hub_off, int64_t n_hub, int64_t n_hub_edges,
-                        int64_t n_band, int band_shift, int32_t thresh, int32_t min_run, int32_t* band_plan, void* ws,
-                        size_t ws_bytes, void* stream) {
+int gmlm_hub_band_order(const int32_t* hub_col, const int32_t* rank, const int32_t* hub_off, int64_t n_hub,
+                        int64_t n_hub_edges, int64_t n_band, int band_shift, int32_t thresh, int32_t min_run,
+                        int32_t* band_plan, void* ws, size_t ws_bytes, void* stream) {
   GMLM_REQUIRE(n_hub >= 0 && n_band >= n_hub && n_band <= n_hub_edges, "hub_band_order: bad sizes");
   GMLM_REQUIRE(band_shift >= 1 && band_shift <= 30 && thresh >= 1 && min_run >= 1, "hub_band_order: bad band parameters");
   GMLM_REQUIRE(ws_bytes >= gmlm_hub_band_workspace_bytes(n_hub_edges), "hub_band_order: workspace too small");
@@ -719,7 +794,7 @@ int gmlm_hub_band_order(const int32_t* hub_col, const int32_t* hub_off, int64_t 
   void* prim_ws = cv.take<char>(0);
   const size_t prim_bytes = ws_bytes - cv.used();
   hub_band_fill_kernel<<<int((n_hub + 1 + kThreads - 1) / kThreads), kThreads, 0, st>>>(
-      hub_col, hub_off, band_chunk_ptr, n_hub, band_shift, thresh, min_run, cut, keys_a, vals_a);
+      hub_col, rank, hub_off, band_chunk_ptr, n_hub, band_shift, thresh, min_run, cut, keys_a, vals_a);
   GMLM_LAUNCH_CHECK();
   // stable by band: chunks of one band keep their row order
   if (int rc = prim::radix_sort_pairs(keys_a, vals_a, keys_b, order, n_band, bits_for((uint64_t(0x7fffffff) >> band_shift) + 1),

@@ -24,11 +24,12 @@
 //   * chunk kernel (hub path): rows longer than `hub_thresh` are cut into fixed chunks of
 //     hub_thresh edges, one group per chunk, fp32 partials, then an in-order final sum.
 //     Contiguous 512-byte rows (F = 256 bf16 / 128 fp32) run the band-ordered hub plan instead
-//     (gmlm_hub_band_sort): each hub row's edges sorted by source, chunks also cut where the
-//     source crosses a band of 2^17 rows, and the chunks launched band by band (chunk_order),
-//     so the rows of one band are gathered from L2 while that band's chunks run.
+//     (gmlm_hub_band_sort): each hub row's edges sorted by the use rank of the gathered row
+//     (gmlm_col_rank), chunks also cut where the rank crosses a band of 2^16 rows, and the chunks
+//     launched band by band (chunk_order), so the rows of one band are gathered from L2 while
+//     that band's chunks run.
 //   * Determinism: fp32 accumulation in a fixed order (CSR order = original edge order; hub rows
-//     of the band plan in source order), fixed chunking, no atomics: bit-identical run to run.
+//     of the band plan in rank order), fixed chunking, no atomics: bit-identical run to run.
 #include <cuda.h>
 
 #include <algorithm>
@@ -967,7 +968,7 @@ extern "C" int gmlm_spmm_csr_banded(const void* x, int dtype, int64_t feat, int6
   q.w_stride = w_heads; q.slab_stride = head_width; q.slab_width = head_width;
   q.n_chunks = n_chunks; q.out = hub_ws; q.order = nullptr;
   // Contiguous rows of exactly 512 bytes, one weight column: the hub chunks of the band plan, run band by band, so
-  // that the rows one band of sources holds are gathered from L2 (DESIGN 4.1); a hub row is then summed in source
+  // that the rows one band of gathered rows holds come from L2 (DESIGN 4.1); a hub row is then summed in band-key
   // order.  Every other width runs the CSR-order chunks of the hub plan.
   const bool banded = band_plan && n_hub > 0 && (mode != GMLM_AGG_WEIGHTED || hub_w) && aligned &&
                       feat * esz == 512 && ldx == feat && w_heads == 1;

@@ -21,11 +21,12 @@ from . import _lib
 
 DEFAULT_HUB_THRESH = int(os.environ.get("GMLM_HUB_THRESH", "256"))
 DEFAULT_QUANTUM = int(os.environ.get("GMLM_GROUP_QUANTUM", "512"))   # 0 = uniform 32-row groups
-# Band-ordered hub plan (gmlm_hub_band_sort): a band is 2^HUB_BAND_SHIFT source rows, 64 MB of 512-byte rows, half
-# of the 126 MB L2.  Of 2^15 / 2^16 / 2^17 rows, 2^17 gave the fastest hub kernels on the C5 and C4 graphs
-# (DESIGN §4.1, profiles/r4_time_hub_chunks.jsonl).  A band boundary splits a chunk only when both pieces keep
-# HUB_BAND_MIN_RUN edges: shorter pieces cost a partial row written and read for few gathered rows.
-HUB_BAND_SHIFT = 17
+# Band-ordered hub plan (gmlm_hub_band_sort), keyed on the use rank of the gathered rows: a band is the next
+# 2^HUB_BAND_SHIFT rows by use, 32 MB of 512-byte rows.  Of 2^16 / 2^17 / 2^18 rows, 2^16 gave the fastest hub
+# kernels on the C5 and C4 graphs in both directions (DESIGN §4.1, profiles/r7_time_hub_chunks.jsonl).  A band
+# boundary splits a chunk only when both pieces keep HUB_BAND_MIN_RUN edges: shorter pieces cost a partial row
+# written and read for few gathered rows.
+HUB_BAND_SHIFT = 16
 HUB_BAND_MIN_RUN = 32
 
 
@@ -58,7 +59,7 @@ class CSR:
     hub_chunk_ptr: Optional[torch.Tensor] = None
     chunk_beg: Optional[torch.Tensor] = None
     chunk_end: Optional[torch.Tensor] = None
-    hub_col: Optional[torch.Tensor] = None     # int32 [hub edges] col of the hub rows, each row sorted by source
+    hub_col: Optional[torch.Tensor] = None     # int32 [hub edges] col of the hub rows, each row sorted by band key
     hub_w: Optional[torch.Tensor] = None       # float32 [hub edges] w in the same order (weighted CSRs)
     band_plan: Optional[torch.Tensor] = None   # int32 [band_chunk_ptr | cut | chunk_order] (include/gmlm_b200.h)
     quantum: int = 0                           # cost-balanced group plan (0 = uniform groups)
@@ -117,8 +118,22 @@ class CSR:
                                              _stream(dev)), "hub_fill")
             else:
                 self.hub_row = self.hub_chunk_ptr = self.chunk_beg = self.chunk_end = None
-        self.plan_bands()
+        self.plan_bands(rank=self.col_rank() if self.n_hub else None)
         return self
+
+    def col_rank(self) -> torch.Tensor:
+        """int32 [max(col) + 1]: rank of every gathered row by the number of edges that gather it, most-gathered
+        first, ties by ascending id (``gmlm_col_rank``)."""
+        lib = _lib.load()
+        dev = self.rowptr.device
+        num_cols = int(self.col.max().item()) + 1 if self.nnz else 0
+        with torch.cuda.device(dev):
+            rank = torch.empty(num_cols, dtype=torch.int32, device=dev)
+            ws_bytes = lib.gmlm_col_rank_workspace_bytes(num_cols)
+            ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+            _lib.check(lib.gmlm_col_rank(_ptr(self.col), self.nnz, num_cols, _ptr(rank), _ptr(ws), ws_bytes,
+                                         _stream(dev)), "col_rank")
+        return rank
 
     @property
     def n_band_chunks(self) -> int:
@@ -126,9 +141,11 @@ class CSR:
             return 0
         return (int(self.band_plan.numel()) - self.n_hub - 2) // 2
 
-    def plan_bands(self, band_shift: int = HUB_BAND_SHIFT):
-        """The band-ordered hub plan next to the hub plan: every hub row's edges sorted by source, cut into chunks
-        at most ``hub_thresh`` long and at band boundaries, chunks ordered by band (``gmlm_hub_band_*``)."""
+    def plan_bands(self, band_shift: int = HUB_BAND_SHIFT, rank: Optional[torch.Tensor] = None):
+        """The band-ordered hub plan next to the hub plan: every hub row's edges sorted by band key, cut into chunks
+        at most ``hub_thresh`` long and at band boundaries, chunks ordered by band (``gmlm_hub_band_*``).  The key
+        of a gathered row is ``rank[row]`` (``col_rank()``: band 0 holds the most-gathered rows, as ``plan_hubs``
+        builds it), or the row id when ``rank`` is None."""
         self.hub_col = self.hub_w = self.band_plan = None
         if not self.n_hub:
             return self
@@ -147,16 +164,16 @@ class CSR:
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
             n_band = C.c_int64(0)
             _lib.check(lib.gmlm_hub_band_sort(_ptr(self.rowptr), _ptr(self.col), _ptr(self.w if hub_w is not None else None),
-                                              self.n_hub, _ptr(self.hub_row), _ptr(hub_off), n_edges, int(band_shift),
-                                              self.hub_thresh, HUB_BAND_MIN_RUN, _ptr(hub_col), _ptr(hub_w),
-                                              _ptr(chunk_ptr), C.byref(n_band), _ptr(ws), ws_bytes, _stream(dev)),
-                       "hub_band_sort")
+                                              _ptr(rank), self.n_hub, _ptr(self.hub_row), _ptr(hub_off), n_edges,
+                                              int(band_shift), self.hub_thresh, HUB_BAND_MIN_RUN, _ptr(hub_col),
+                                              _ptr(hub_w), _ptr(chunk_ptr), C.byref(n_band), _ptr(ws), ws_bytes,
+                                              _stream(dev)), "hub_band_sort")
             nb = int(n_band.value)
             band_plan = torch.empty(self.n_hub + 2 + 2 * nb, dtype=torch.int32, device=dev)
             band_plan[:self.n_hub + 1].copy_(chunk_ptr)
-            _lib.check(lib.gmlm_hub_band_order(_ptr(hub_col), _ptr(hub_off), self.n_hub, n_edges, nb, int(band_shift),
-                                               self.hub_thresh, HUB_BAND_MIN_RUN, _ptr(band_plan), _ptr(ws), ws_bytes,
-                                               _stream(dev)), "hub_band_order")
+            _lib.check(lib.gmlm_hub_band_order(_ptr(hub_col), _ptr(rank), _ptr(hub_off), self.n_hub, n_edges, nb,
+                                               int(band_shift), self.hub_thresh, HUB_BAND_MIN_RUN, _ptr(band_plan),
+                                               _ptr(ws), ws_bytes, _stream(dev)), "hub_band_order")
         self.hub_col, self.hub_w, self.band_plan = hub_col, hub_w, band_plan
         return self
 

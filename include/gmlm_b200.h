@@ -127,25 +127,34 @@ int gmlm_hub_fill(const int32_t* rowptr, int64_t num_rows, int32_t thresh, int64
                   int32_t* hub_row, int32_t* hub_chunk_ptr, int32_t* chunk_beg, int32_t* chunk_end,
                   void* ws, size_t ws_bytes, void* stream);
 
+/* ---- use rank of gathered rows (the band key of the hub plan below) ----
+ * rank[num_cols]: rank[c] = position of row c when the rows are ordered by the number of edges of col[nnz] that
+ * gather them, most-gathered first, ties by ascending id; rows no edge gathers come last.  A permutation of
+ * [0, num_cols).  Fails with GMLM_ERR_INDEX when col holds a value outside [0, num_cols) (synchronises). */
+size_t gmlm_col_rank_workspace_bytes(int64_t num_cols);
+int gmlm_col_rank(const int32_t* col, int64_t nnz, int64_t num_cols, int32_t* rank, void* ws, size_t ws_bytes,
+                  void* stream);
+
 /* ---- band-ordered hub plan (512-byte rows of gmlm_spmm_csr_banded) ----
- * The edges of every hub row sorted by source (stable: ties keep CSR order), so that the chunks gathering from one
- * band of 2^band_shift source rows can run together and find those rows in L2.
+ * The edges of every hub row sorted by band key (stable: ties keep CSR order), so that the chunks gathering from one
+ * band of 2^band_shift keys can run together and find those rows in L2.  The key of gathered row c is rank[c]
+ * (gmlm_col_rank of the same CSR: band 0 holds the most-gathered rows), or c itself when rank is NULL.
  * hub_off[n_hub+1]: hub_off[h] = edges of hub rows before h (exclusive scan of the hub row lengths).
  * band_sort : hub_col[n_hub_edges] (and hub_w, when w is given) = col / w of the hub rows, row by row, each row by
- *             source; band_chunk_ptr[n_hub+1] = the row -> chunk pointer of the band cuts; *n_band_host = #chunks.
+ *             key; band_chunk_ptr[n_hub+1] = the row -> chunk pointer of the band cuts; *n_band_host = #chunks.
  *             A band boundary inside a row is a cut when both sides hold >= min_run edges; pieces between cuts are
  *             cut every `thresh` edges.
  * band_order: band_plan = [band_chunk_ptr (n_hub+1, copied in by the caller) | cut (n_band+1) | chunk_order (n_band)];
  *             chunk c covers hub_col[cut[c], cut[c+1]); chunk_order = chunk ids stably sorted by the band of their
- *             first edge. */
+ *             first edge.  rank must be the one band_sort was given. */
 size_t gmlm_hub_band_workspace_bytes(int64_t n_hub_edges);
-int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w, int64_t n_hub, const int32_t* hub_row,
-                       const int32_t* hub_off, int64_t n_hub_edges, int band_shift, int32_t thresh, int32_t min_run,
-                       int32_t* hub_col, float* hub_w, int32_t* band_chunk_ptr, int64_t* n_band_host, void* ws,
-                       size_t ws_bytes, void* stream);
-int gmlm_hub_band_order(const int32_t* hub_col, const int32_t* hub_off, int64_t n_hub, int64_t n_hub_edges,
-                        int64_t n_band, int band_shift, int32_t thresh, int32_t min_run, int32_t* band_plan, void* ws,
-                        size_t ws_bytes, void* stream);
+int gmlm_hub_band_sort(const int32_t* rowptr, const int32_t* col, const float* w, const int32_t* rank, int64_t n_hub,
+                       const int32_t* hub_row, const int32_t* hub_off, int64_t n_hub_edges, int band_shift,
+                       int32_t thresh, int32_t min_run, int32_t* hub_col, float* hub_w, int32_t* band_chunk_ptr,
+                       int64_t* n_band_host, void* ws, size_t ws_bytes, void* stream);
+int gmlm_hub_band_order(const int32_t* hub_col, const int32_t* rank, const int32_t* hub_off, int64_t n_hub,
+                        int64_t n_hub_edges, int64_t n_band, int band_shift, int32_t thresh, int32_t min_run,
+                        int32_t* band_plan, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- cost-balanced group plan for gmlm_spmm_csr ----
  * Cuts the row sequence where (r + rowptr[r]) crosses multiples of `quantum`, so that every

@@ -1,9 +1,11 @@
 """Time the hub path of the aggregation alone (chunk_kernel + hub_final_kernel, from torch.profiler kernel records)
-on the C5 / C4 graphs, forward (mean) and backward (weighted), for the CSR-order chunk plan and the band-ordered plan
-at several band shifts and hub thresholds.  Next to each time: the modelled gather traffic of the band plan (distinct
-source rows per band pass x 512 bytes, against one row per hub edge), a model and not a DRAM measurement.
+and the whole call (every kernel of it) on the C5 / C4 graphs, forward (mean) and backward (weighted), for the
+CSR-order chunk plan and the band-ordered plan keyed on the gathered row id ("id") or on its use rank ("rank",
+CSR.col_rank) at several band shifts and hub thresholds.  Next to each time: the modelled gather traffic of the band
+plan (distinct gathered rows per band pass x 512 bytes, against one row per hub edge), a model and not a DRAM
+measurement.
 
-    python tools/time_hub_chunks.py [--graphs c5 c4] [--iters 10] [--out profiles/x.jsonl]
+    python tools/time_hub_chunks.py [--graphs c5 c4] [--keys id rank] [--iters 10] [--out profiles/x.jsonl]
 """
 from __future__ import annotations
 
@@ -25,28 +27,33 @@ HUB_KERNELS = ("chunk_kernel", "hub_final_kernel")
 
 
 def hub_ms(fn, iters):
-    """Mean ms per call of the hub kernels of `fn` (kernel records of torch.profiler)."""
+    """Mean ms per call of the hub kernels of `fn` and of all its kernels ("call") (kernel records of
+    torch.profiler)."""
     fn()
     torch.cuda.synchronize()
     with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
         for _ in range(iters):
             fn()
         torch.cuda.synchronize()
-    tot = {k: 0.0 for k in HUB_KERNELS}
+    tot = {k: 0.0 for k in HUB_KERNELS + ("call",)}
     for ev in prof.events():
+        t = ev.device_time_total if hasattr(ev, "device_time_total") else ev.cuda_time_total
+        if ev.device_type == torch.autograd.DeviceType.CUDA:
+            tot["call"] += t
         for k in HUB_KERNELS:
             if k in ev.name and "tma" not in ev.name:
-                tot[k] += ev.device_time_total if hasattr(ev, "device_time_total") else ev.cuda_time_total
+                tot[k] += t
     return {k: v / iters / 1e3 for k, v in tot.items()}
 
 
-def gather_model(csr, shift):
-    """Hub edges and distinct source rows per band pass (chunks grouped by the band of their first edge)."""
+def gather_model(csr, shift, rank):
+    """Hub edges and distinct gathered rows per band pass (chunks grouped by the band of their first edge)."""
     nh, nb = csr.n_hub, csr.n_band_chunks
     bp = csr.band_plan.long()
     cut = bp[nh + 1:nh + 2 + nb]
     lens = cut[1:] - cut[:-1]
-    first_band = csr.hub_col.long()[cut[:-1]] >> shift
+    band_key = csr.hub_col.long() if rank is None else rank.long()[csr.hub_col.long()]
+    first_band = band_key[cut[:-1]] >> shift
     band_of_edge = torch.repeat_interleave(first_band, lens)
     key = band_of_edge * (int(csr.hub_col.max().item()) + 1) + csr.hub_col.long()
     distinct = int(torch.unique(key).numel())
@@ -64,7 +71,8 @@ def without_bands(csr):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--graphs", nargs="+", default=["c5", "c4"])
-    ap.add_argument("--shifts", nargs="+", type=int, default=[15, 16, 17])
+    ap.add_argument("--shifts", nargs="+", type=int, default=[16, 17, 18])
+    ap.add_argument("--keys", nargs="+", default=["id", "rank"], choices=["id", "rank"])
     ap.add_argument("--threshs", nargs="+", type=int, default=[256, 128, 64])
     ap.add_argument("--iters", type=int, default=10)
     ap.add_argument("--out", default=None)
@@ -98,19 +106,26 @@ def main():
                 emit({"graph": key, "dir": name, "hub_thresh": thresh, "plan": "csr_order",
                       "ms": hub_ms(lambda: G.spmm(inp, plain, mode, out=buf), args.iters),
                       "hub_rows": csr.n_hub, "chunks": csr.n_chunks})
-                for shift in (args.shifts if thresh == args.threshs[0] else [HUB_BAND_SHIFT]):
-                    torch.cuda.synchronize()
-                    t0 = time.perf_counter()
-                    csr.plan_bands(shift)
-                    torch.cuda.synchronize()
-                    t_plan = time.perf_counter() - t0
-                    d = {"graph": key, "dir": name, "hub_thresh": thresh, "plan": "banded", "band_shift": shift,
-                         "ms": hub_ms(lambda: G.spmm(inp, csr, mode, out=buf), args.iters), "plan_build_s": t_plan,
-                         "plan_bytes": 4 * (csr.hub_col.numel() + csr.band_plan.numel()) +
-                         (4 * csr.hub_w.numel() if csr.hub_w is not None else 0)}
-                    d.update(model=gather_model(csr, shift))
-                    emit(d)
-                csr.plan_bands()
+                for band_key in args.keys:
+                    for shift in (args.shifts if thresh == args.threshs[0] else [HUB_BAND_SHIFT]):
+                        torch.cuda.synchronize()
+                        t0 = time.perf_counter()
+                        rank = csr.col_rank() if band_key == "rank" else None
+                        torch.cuda.synchronize()
+                        t_rank = time.perf_counter() - t0
+                        csr.plan_bands(shift, rank=rank)
+                        torch.cuda.synchronize()
+                        t_plan = time.perf_counter() - t0
+                        d = {"graph": key, "dir": name, "hub_thresh": thresh, "plan": "banded", "band_key": band_key,
+                             "band_shift": shift, "ms": hub_ms(lambda: G.spmm(inp, csr, mode, out=buf), args.iters),
+                             "plan_build_s": t_plan, "rank_build_s": t_rank,
+                             "plan_bytes": 4 * (csr.hub_col.numel() + csr.band_plan.numel()) +
+                             (4 * csr.hub_w.numel() if csr.hub_w is not None else 0),
+                             "rank_bytes": 4 * rank.numel() if rank is not None else 0}
+                        d.update(model=gather_model(csr, shift, rank))
+                        emit(d)
+                        del rank
+                csr.plan_hubs(csr.hub_thresh)
             for csr in (g.fwd, g.bwd):
                 csr.plan_hubs(G.graph.DEFAULT_HUB_THRESH)
         del g, ei, et, x, gh, h_buf, gx_buf
