@@ -53,7 +53,7 @@ def test_dst_plan_matches_numpy_restatement(cuda_dev):
 
 
 @pytest.mark.parametrize("n,e,fi,fo", [(183, 300, 1703, 64), (3000, 40000, 256, 64), (500, 6000, 96, 32),
-                                      (500, 6000, 96, 22), (1, 2, 16, 8)])
+                                      (500, 6000, 96, 22), (1, 2, 16, 8), (3000, 40000, 512, 128)])
 def test_transform_first_fp32_matches_oracle_and_aggregate_first(cuda_dev, n, e, fi, fo):
     torch.manual_seed(1)
     ei = synth.rmat_edges(n, e, seed=n) if n > 1 else torch.zeros(2, e, dtype=torch.int64)
@@ -86,7 +86,17 @@ def test_transform_first_fp32_matches_oracle_and_aggregate_first(cuda_dev, n, e,
 
 def test_transform_first_bf16_tcgen05_matches_oracle(cuda_dev):
     """The bandwidth-study input layer (256 -> 64, bf16): Z on the tcgen05 GEMM, 128-byte slab gather."""
-    n, e, fi, fo = 5000, 90000, 256, 64
+    _bf16_transform_first_matches_oracle(cuda_dev, 256, 64)
+
+
+def test_transform_first_bf16_tcgen05_512B_slabs_match_oracle(cuda_dev):
+    """1024 -> 256, bf16: the gathered slabs are 512-byte rows, whose hub rows take the band plan (weighted, with
+    hub_w)."""
+    _bf16_transform_first_matches_oracle(cuda_dev, 1024, 256)
+
+
+def _bf16_transform_first_matches_oracle(cuda_dev, fi, fo):
+    n, e = 5000, 90000
     torch.manual_seed(0)
     ei = synth.rmat_edges(n, e, seed=3)
     et = edge_type_bucket_ref(ei, n)
